@@ -4,6 +4,7 @@ human36, fp64, dt = 1 ms).
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # reference CPU path (oracle port)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # ... and the state after the last timed step
 
 A "step" is one pass of the hot path (update_dynamic -> update_controllers ->
 update_constraints -> integrate) over the whole batch of worlds.  Prints ONE JSON
@@ -45,6 +46,7 @@ GROUPS = 10        # the batch is split into GROUPS contiguous blocks whose epis
 PHASE = EPISODE//GROUPS   # by PHASE steps, so that at ANY step the batch holds every age of the
                    # episode (free fall, first contacts, 8 contacts with ~20 % sliding) in equal
                    # shares: the measured rate does not depend on which steps are timed
+DUMP_BYTES = 32 << 20      # --dump-outputs: at most this many bytes of arrays (well under 64 MB)
 
 
 # ---------------------------------------------------------------------------------------
@@ -102,7 +104,18 @@ def parse():
                     help="serial mode: 'priority' = one compute stream per block, earlier blocks at higher "
                          "priority (default); N = N plain streams")
     ap.add_argument("--opt", action="append", help="arb_batch_set_option switch, name=value (A/B runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the state they leave (gpos, gvel, cforce) of a fixed, "
+                         "seeded sample of rank 0's worlds to DIR/<name>.npy (float64, %d MB of arrays at "
+                         "most), with the sampled world indices in DIR/world.npy; worlds whose state is not "
+                         "finite are left out of the sample and listed in DIR/nonfinite_world.npy"
+                         % (DUMP_BYTES >> 20))
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def config_of(a, scen, total, per_gpu, world_size, scaling, model=None):
@@ -278,6 +291,38 @@ def parity_sample(bw, model, scen, nsample=8):
                    "same state (checker only, not timed)"}
 
 
+def dump_sample(W, model):
+    """Indices (ascending) of the worlds of a W-world batch whose state --dump-outputs writes: all of
+    them when their state fits DUMP_BYTES, otherwise a fixed, seeded sample that does."""
+    per_world = 8*(int(model.ngpos) + int(model.ndof) + int(model.nrows) + 1)     # + its index
+    n = min(W, DUMP_BYTES//per_world)
+    return np.sort(np.random.default_rng(0).choice(W, size=n, replace=False))
+
+
+def sample_outputs(bw, model, w0):
+    """What a caller of the timed step reads back (BatchedWorld.get_state: gpos, gvel, cforce as
+    (elem, worlds) float64) for the worlds of dump_sample whose state is finite, and their indices in
+    the whole batch.  A world whose state is not finite has no result to compare: the reference's own
+    algorithm diverges there (profiles/README.md).  Those worlds of the whole batch are listed by index
+    instead ("nonfinite_world", only when there are any)."""
+    import torch
+    state = {"gpos": bw.gpos, "gvel": bw.gvel}
+    if model.nrows:
+        state["cforce"] = bw.cforce[:int(model.nrows)]
+    finite = torch.ones(bw.nworlds, dtype=torch.bool, device=bw.gpos.device)
+    for t in state.values():
+        finite &= torch.isfinite(t).all(0)
+    finite = finite.cpu().numpy()
+    ids = dump_sample(bw.nworlds, model)
+    ids = ids[finite[ids]]
+    idx = torch.as_tensor(ids, device=bw.gpos.device)
+    out = {name: t[:, idx].cpu().numpy() for name, t in state.items()}
+    out["world"] = (ids + w0).astype(np.float64)
+    if not finite.all():
+        out["nonfinite_world"] = (np.flatnonzero(~finite) + w0).astype(np.float64)
+    return out
+
+
 def measure(a, scen, model, w0, w1, rank, world_size, local, full):
     """Time `a.steps` steps of worlds [w0, w1) on this rank's GPU.  Returns a dict of raw numbers
     (before the reduction over ranks).  `full`: also stage times, active-set mix, parity sample."""
@@ -317,12 +362,19 @@ def measure(a, scen, model, w0, w1, rank, world_size, local, full):
     barrier()
     ms = e0.elapsed_time(e1)
     launches = bw.launch_count() - l0
+    dump = None
+    if a.dump_outputs and full and rank == 0:     # before anything below steps the batch further
+        dump = sample_outputs(bw, model, w0)
     if not sampler.rows:            # a very short timed region: keep the load up until one sample exists
         t_end = time.time() + 10.
         while not sampler.rows and time.time() < t_end:
             ep.advance(PHASE)
             torch.cuda.synchronize()
     sampler.stop_flag = True
+    if dump is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, v in dump.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), v)
     bad = (~torch.isfinite(bw.gvel)).any(0)
     nonfinite = int(bad.sum())
     out = {"W": W, "ms": ms, "launches": launches, "nonfinite": nonfinite, "warm": warm,

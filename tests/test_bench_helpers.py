@@ -1,9 +1,12 @@
 """bench.py's host-side helpers: the SURVEY.md 8(d) flop formulas (pinned to the survey's own
-worked numbers) and the config object both arms print."""
+worked numbers), the config object both arms print, and what --dump-outputs writes."""
+import json
 import os
+import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -74,3 +77,70 @@ def test_traffic_json_follows_from_the_committed_ncu_summaries():
         tot_f += f
     assert abs(doc["dram_bytes_per_world_step"] - tot_b) <= 1e-9*tot_b
     assert abs(doc["executed_fp64_flop_per_world_step"] - tot_f) <= 1e-9*tot_f
+
+
+def test_dump_sample_is_fixed_and_bounded():
+    """--dump-outputs writes the same worlds every run: a seeded sample below 64 MB at the bench size,
+    the whole batch when it fits."""
+    m = flatten(scenarios.human36_contact_world())
+    ids = bench.dump_sample(262144, m)
+    assert np.array_equal(ids, bench.dump_sample(262144, m))
+    assert ids[0] >= 0 and ids[-1] < 262144 and (np.diff(ids) > 0).all()
+    assert len(ids)*8*(m.ngpos + m.ndof + m.nrows + 1) <= bench.DUMP_BYTES < 64 << 20
+    assert np.array_equal(bench.dump_sample(640, m), np.arange(640))
+
+
+def test_dump_leaves_out_worlds_without_a_finite_state():
+    """A world whose state is not finite (the reference's own algorithm diverges there) is not part
+    of the dumped sample; every such world of the batch is listed by index instead."""
+    import torch
+    m = flatten(scenarios.human36_contact_world())
+    W, w0 = 300, 1000
+
+    class Batch(object):          # the state tensors of a BatchedWorld, on the host
+        nworlds = W
+        gpos = torch.rand(m.ngpos, W, dtype=torch.float64)
+        gvel = torch.rand(m.ndof, W, dtype=torch.float64)
+        cforce = torch.rand(m.nrows, W, dtype=torch.float64)
+    Batch.gvel[3, 17] = float("nan")
+    Batch.gpos[0, 250] = float("inf")
+    Batch.cforce[m.nrows - 1, 5] = float("nan")
+    out = bench.sample_outputs(Batch, m, w0)
+    keep = [w for w in range(W) if w not in (5, 17, 250)]
+    assert np.array_equal(out["world"], np.array(keep) + w0)
+    assert np.array_equal(out["nonfinite_world"], [w0 + 5, w0 + 17, w0 + 250])
+    for name in ("gpos", "gvel", "cforce"):
+        assert np.array_equal(out[name], getattr(Batch, name)[:, keep].numpy())
+    assert all(v.dtype == np.float64 and np.isfinite(v).all() for v in out.values())
+    Batch.gvel[3, 17] = Batch.gpos[0, 250] = Batch.cforce[m.nrows - 1, 5] = 0.
+    assert "nonfinite_world" not in bench.sample_outputs(Batch, m, w0)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_state_after_the_timed_steps(tmp_path):
+    """bench.py --dump-outputs writes the state its last timed step leaves: bit for bit that of the
+    same worlds stepped here through the same staggered episodes, warm-up then --steps steps."""
+    import torch
+    from arboris_b200.batch import BatchedWorld
+    W, warm, steps = 640, 4, 7
+    run = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--worlds", str(W),
+                          "--steps", str(steps), "--warmup", str(warm), "--no-e2e", "--no-cpu-baseline",
+                          "--no-parity-sample", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, check=True)
+    line = json.loads(run.stdout.strip().splitlines()[-1])
+    assert line["steps"] == steps and line["warmup"] == warm and line["config"]["worlds_total"] == W
+    scen = bench.WORKLOADS[line["config"]["workload"]][0]
+    model = flatten(scenarios.BUILDERS[scen]())
+    gp, gv = scenarios.initial_states(model, scen, 0, W)
+    bw = BatchedWorld(model, W, device="cuda:0")
+    ep = bench.Episodes(W, (bw.gpos, bw.gvel, bw.cforce),
+                        (torch.as_tensor(gp, device=bw.device), torch.as_tensor(gv, device=bw.device), None),
+                        lambda c: bw.step(bench.DT, c))
+    ep.prime()
+    ep.advance(warm)
+    ep.advance(steps)
+    g, v, f = bw.get_state()
+    got = {name: np.load(str(tmp_path/(name + ".npy"))) for name in ("gpos", "gvel", "cforce", "world")}
+    assert all(x.dtype == np.float64 for x in got.values())
+    assert np.array_equal(got["world"], np.arange(W))
+    assert np.array_equal(got["gpos"], g) and np.array_equal(got["gvel"], v) and np.array_equal(got["cforce"], f)
