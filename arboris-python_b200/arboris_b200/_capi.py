@@ -85,6 +85,7 @@ SYMBOLS = [
     ("arb_batch_bind_state", _i32, [_vp, _vp, _vp, _vp]),
     ("arb_batch_bind_controller_params", _i32, [_vp, _vp, _vp, _vp, _vp]),
     ("arb_model_pd_dofs", _i32, [_vp, c_i32p, _i32]),
+    ("arb_batch_bind_applied_forces", _i32, [_vp, _vp, _i32, c_i32p, _vp]),
     ("arb_batch_step_path", _i32, [_vp, C.POINTER(C.c_char_p)]),
     ("arb_update_dynamic", _i32, [_vp]),
     ("arb_update_controllers", _i32, [_vp, _dbl]),

@@ -64,6 +64,8 @@ class BatchedWorld(object):
         self._current_time = 0.
         self._pinned = None
         self._ctrl_params = {}
+        self.applied_gforce = self.applied_wrench = None
+        self.applied_bodies = ()
         why = C.c_char_p()
         if self._lib.arb_batch_step_path(self._batch_h, C.byref(why)) == 0:
             # not silent: the fused stages fold controllers per dof; anything else runs the
@@ -151,6 +153,49 @@ class BatchedWorld(object):
         ptr = [self._ctrl_params[k].data_ptr() if k in self._ctrl_params else None
                for k in ("kp", "kd", "gpos_des", "gvel_des")]
         _capi.check(self._lib, self._lib.arb_batch_bind_controller_params(self._batch_h, *ptr))
+
+    # ---- per-world applied forces --------------------------------------------------------------
+    def set_applied_forces(self, gforce=None, wrench=None, bodies=None):
+        """Per-world forces of a controller added after the model's ones (what a reference
+        ``Controller`` whose ``update`` returns ``(gforce, 0)`` adds):
+
+        ``gforce``: (ndof, W) generalized forces;  ``wrench``: (len(bodies), 6, W) wrenches
+        [torque; force] in ground axes acting at the origin of body ``bodies[i]`` (indices as in
+        ``body()``, the ground excluded).  Numpy or torch; ``None`` keeps what is bound (``bodies``
+        too), ``False`` unbinds (a wrench and its bodies together).  The bound fp64 device tensors
+        are ``applied_gforce`` and ``applied_wrench`` (the argument itself when it already is one):
+        write into them in place to change the forces between steps without another call."""
+        W = self.nworlds
+
+        def dev(v, shape, name):
+            t = torch.as_tensor(np.ascontiguousarray(v) if isinstance(v, np.ndarray) else v,
+                                dtype=torch.float64).to(self.device).contiguous()
+            if tuple(t.shape) != shape:
+                raise ValueError("%s must have shape %s, not %s" % (name, shape, tuple(t.shape)))
+            return t
+
+        g, wr, bd = self.applied_gforce, self.applied_wrench, self.applied_bodies
+        if gforce is False:
+            g = None
+        elif gforce is not None:
+            g = dev(gforce, (self.ndof, W), "gforce")
+        if wrench is False:
+            wr, bd = None, ()
+        else:
+            if bodies is not None:
+                bd = tuple(int(b) for b in np.asarray(bodies).reshape(-1))
+            if wrench is not None:
+                wr = dev(wrench, (len(bd), 6, W), "wrench")
+            elif wr is not None and tuple(wr.shape) != (len(bd), 6, W):
+                raise ValueError("the bound wrench has %d bodies, not %d: pass the wrench with its bodies"
+                                 % (wr.shape[0], len(bd)))
+        ids = (C.c_int32*max(len(bd), 1))(*bd)
+        self._sync_stream()         # (the body table is replaced in stream order)
+        _capi.check(self._lib, self._lib.arb_batch_bind_applied_forces(
+            self._batch_h, g.data_ptr() if g is not None else None, len(bd) if wr is not None else 0,
+            ids, wr.data_ptr() if wr is not None else None))
+        self.applied_gforce, self.applied_wrench = g, wr
+        self.applied_bodies = bd if wr is not None else ()
 
     # ---- the four phases and the fused step ---------------------------------------------
     def update_dynamic(self):

@@ -162,6 +162,7 @@ extern "C" void arb_batch_destroy(arb_batch* b) {
   cudaFree(b->scratch_dbl);
   cudaFree(b->scratch_int);
   cudaFree(b->d.status);
+  cudaFree(b->applied_rows);
   arb_fused_release(b);
   delete b;
 }
@@ -214,6 +215,26 @@ extern "C" int arb_batch_bind_controller_params(arb_batch* b, const double* kp, 
   return 0;
 }
 
+extern "C" int arb_batch_bind_applied_forces(arb_batch* b, const double* gforce, int nbodies, const int32_t* bodies,
+                                             const double* wrench) {
+  if (!b) { arb_set_error("null batch"); return -1; }
+  std::vector<int> rows;
+  std::string err;
+  if (applied_wrench_rows(b->model->host, nbodies, bodies, wrench != nullptr, rows, err)) {
+    arb_set_error(err);
+    return -1;
+  }
+  CUDA_OK(cudaSetDevice(b->device));
+  if (!b->applied_rows) CUDA_OK(cudaMalloc((void**)&b->applied_rows, sizeof(int) * rows.size()));
+  // in stream order: the steps already enqueued read the previous table
+  CUDA_OK(cudaMemcpyAsync(b->applied_rows, rows.data(), sizeof(int) * rows.size(), cudaMemcpyHostToDevice, b->stream));
+  CUDA_OK(cudaStreamSynchronize(b->stream));
+  b->applied.tau = gforce;
+  b->applied.wrench = nbodies > 0 ? wrench : nullptr;
+  b->applied.row = b->applied_rows;
+  return 0;
+}
+
 /* 1: arb_step runs the fused stages; 0: it runs the four phase kernels (a controller couples dofs
  * in a way the fused stages do not fold, or "force_phases" is set); *why (optional) names the reason */
 extern "C" int arb_batch_step_path(const arb_batch* b, const char** why) {
@@ -238,9 +259,9 @@ __global__ void __launch_bounds__(LPW_THREADS) k_update_dynamic(DevModel m, DevB
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (w < b.W) world_update_dynamic(m, b, w);
 }
-__global__ void __launch_bounds__(LPW_THREADS) k_update_controllers(DevModel m, DevBatch b, double dt) {
+__global__ void __launch_bounds__(LPW_THREADS) k_update_controllers(DevModel m, DevBatch b, double dt, DevApplied ap) {
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (w < b.W) world_update_controllers(m, b, w, dt);
+  if (w < b.W) world_update_controllers(m, b, w, dt, ap);
 }
 __global__ void __launch_bounds__(LPW_THREADS) k_update_constraints(DevModel m, DevBatch b, double dt) {
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -278,7 +299,7 @@ extern "C" int arb_update_controllers(arb_batch* b, double dt) {
   if (!(dt > 0)) { arb_set_error("dt must be > 0"); return -3; }
   CUDA_OK(cudaSetDevice(b->device));
   rc = arb_ensure_phase_scratch(b); if (rc) return rc;
-  k_update_controllers<<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt);
+  k_update_controllers<<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->applied);
   LAUNCH_CHECK(b);
   return 0;
 }
@@ -311,7 +332,7 @@ int arb_step_phases(arb_batch* b, const double* dts, int nsteps) {
     const double dt = dts[s];
     if (!(dt > 0)) { arb_set_error("dt must be > 0"); return -3; }
     k_update_dynamic<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d);
-    k_update_controllers<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt);
+    k_update_controllers<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->applied);
     k_update_constraints<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt);
     k_integrate<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt);
     b->launches += 3;

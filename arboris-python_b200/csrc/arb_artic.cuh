@@ -320,8 +320,12 @@ ARB_D double artic_pd_diag(const DevModel& m, const DevBatch& b, int64_t w, int 
 
 // ---------------------------------------------------------------------------------------
 // leaf-to-root pass: elimination of every dof (stores U, LA, LM, 1/d) together with the
-// reduced right-hand side u of the free motion (w_b = M_b (T_b/dt + gravity_b), tau = PD).
-ARB_D bool artic_factor(const DevModel& m, const DevBatch& b, int64_t w, double dt) {
+// reduced right-hand side u of the free motion (w_b = M_b (T_b/dt + gravity_b) + applied wrench,
+// tau = PD + applied generalized force).  APPLIED = false: the instantiation without the applied-force
+// terms, which the fused step runs while none are bound (with them ptxas spills 48 more bytes in the
+// prepare kernel, a cost the unbound step need not pay).
+template <bool APPLIED>
+ARB_D bool artic_factor(const DevModel& m, const DevBatch& b, int64_t w, double dt, const DevApplied& ap) {
   bool ok = true;
   // 1/dt once per world: the 36 M_b/dt per body are mostly 0/dt, which sends the fp64 division
   // through its slow path (a quarter of this stage's instructions before)
@@ -414,6 +418,22 @@ ARB_D bool artic_factor(const DevModel& m, const DevBatch& b, int64_t w, double 
 #pragma unroll
       for (int i = 0; i < 36; ++i) IA[i] += Bb[i];
     }
+    // applied wrench (arb_batch_bind_applied_forces), on massless bodies too: -[R^T torque; R^T force]
+    if (APPLIED && ap.wrench) {
+      const int row = ap.row[j];
+      if (row >= 0) {
+        const double* wp = ap.wrench + (int64_t)(6 * row) * b.W + artic_param_world(b, w);
+        double R[9], wg[6], wr[6];
+#pragma unroll
+        for (int i = 0; i < 9; ++i) R[i] = FT(b.fpose, j * 12 + i);
+#pragma unroll
+        for (int i = 0; i < 6; ++i) wg[i] = arb_ld_state(wp + (int64_t)i * b.W);
+        m3t_mulv(R, wg, wr);
+        m3t_mulv(R, wg + 3, wr + 3);
+#pragma unroll
+        for (int i = 0; i < 6; ++i) beta[i] -= wr[i];
+      }
+    }
     // children's contributions: every child joint c left X^T IA X, X^T IM X, X^T beta in ITS
     // OWN slot (no read-modify-write on the way up), summed here
     for (int c = m.jchild0[j]; c >= 0; c = m.jsib[c]) {
@@ -455,7 +475,9 @@ ARB_D bool artic_factor(const DevModel& m, const DevBatch& b, int64_t w, double 
         LA[i] = ta * dinv;
         LM[i] = tm * dinv;
       }
-      const double u = (artic_tau(m, b, w, k) - sb) * dinv;
+      double tau = artic_tau(m, b, w, k);
+      if (APPLIED && ap.tau) tau += arb_ld_state(ap.tau + (int64_t)k * b.W + artic_param_world(b, w));
+      const double u = (tau - sb) * dinv;
       FT(b.au, k) = u;
       FT(b.adinv, k) = dinv;
 #pragma unroll

@@ -81,10 +81,18 @@ struct FusedState {
 #ifndef FINISH_THREADS
 #define FINISH_THREADS 128
 #endif
-__global__ void __launch_bounds__(PREP_THREADS, PREP_MINBLOCKS) k_fused_prepare_lane(DevModel m, DevBatch b, double dt) {
+template <bool APPLIED>
+__global__ void __launch_bounds__(PREP_THREADS, PREP_MINBLOCKS) k_fused_prepare_lane(DevModel m, DevBatch b, double dt, DevApplied ap) {
   FUSED_SLOT_WORLD();
   if (s >= b.W) return;
-  world_fused_prepare(m, fused_tile_view(b, s), w, dt);
+  world_fused_prepare<APPLIED>(m, fused_tile_view(b, s), w, dt, ap);
+}
+// the instantiation with the applied-force terms only while some are bound
+static void launch_prepare_lane(const arb_batch* b, const DevBatch& d, double dt) {
+  const unsigned grid = (unsigned)((d.W + PREP_THREADS - 1) / PREP_THREADS);
+  if (b->applied.tau || b->applied.wrench)
+    k_fused_prepare_lane<true><<<grid, PREP_THREADS, 0, b->stream>>>(b->m, d, dt, b->applied);
+  else k_fused_prepare_lane<false><<<grid, PREP_THREADS, 0, b->stream>>>(b->m, d, dt, b->applied);
 }
 // Threads per CTA of the Gauss-Seidel kernel: 128 (8.87 ms against 9.01 with 64 and 9.11 with 32 at
 // 262144 worlds; end to end, with seven column blocks on three streams, 1.406e7 world-steps/s against
@@ -207,6 +215,13 @@ __global__ void __launch_bounds__(FUSED_THREADS) k_fused_finish_k(DevModel m, De
 static size_t group_smem_bytes(const arb_batch* b) { return sizeof(double) * (size_t)b->m.gl.total * GROUP_WPC; }
 // the group stage needs its per-world record to fit the SM's shared memory
 static bool group_supported(const arb_batch* b) { return group_smem_bytes(b) <= 227 * 1024; }
+// the group prepare stage has no applied-force term: refused rather than stepping without the forces
+static int group_refuses_applied(const arb_batch* b) {
+  if (!(b->prepare_group && group_supported(b) && (b->applied.tau || b->applied.wrench))) return 0;
+  arb_set_error("the prepare_group option does not support applied forces (arb_batch_bind_applied_forces): "
+                "unbind them or clear the option");
+  return -1;
+}
 
 // private by-slot state <- caller's state (GATHER) or the reverse; one thread per slot and
 // ELEMS_PER_BLOCK_Y elements, the by-slot side coalesced
@@ -299,7 +314,8 @@ static int ensure_fused_scratch(arb_batch* b) {
     }
     b->gs_plain = plain ? 1 : 0;
   }
-  CUDA_OKF(cudaFuncSetAttribute(k_fused_prepare_lane, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_prepare_lane<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_prepare_lane<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
   CUDA_OKF(cudaFuncSetAttribute(k_fused_finish, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
   b->fused = f;
   return 0;
@@ -337,7 +353,9 @@ static int fused_state_sync(arb_batch* b, bool gather) {
 int arb_fused_step(arb_batch* b, const double* dts, int nsteps) {
   for (int s = 0; s < nsteps; ++s)       // before anything is enqueued: a bad dt leaves the state untouched
     if (!(dts[s] > 0)) { arb_set_error("dt must be > 0"); return -3; }
-  int rc = ensure_fused_scratch(b);
+  int rc = group_refuses_applied(b);
+  if (rc) return rc;
+  rc = ensure_fused_scratch(b);
   if (rc) return rc;
   FusedState* f = b->fused;
   const HostModel& h = b->model->host;
@@ -428,7 +446,7 @@ int arb_fused_step(arb_batch* b, const double* dts, int nsteps) {
     if (grp)
       k_fused_prepare_group<<<(unsigned)((W + GROUP_WPC - 1) / GROUP_WPC), GROUP_WPC * ARB_GL, group_smem_bytes(b), b->stream>>>(b->m, d, dt, 0);
     else
-      k_fused_prepare_lane<<<(unsigned)((W + PREP_THREADS - 1) / PREP_THREADS), PREP_THREADS, 0, b->stream>>>(b->m, d, dt);
+      launch_prepare_lane(b, d, dt);
     if (ev[0]) cudaEventRecord(ev[1], b->stream);
     if (b->m.nc > 0) {
       if (b->m.nc <= 64 && b->gs_coop)
@@ -464,7 +482,9 @@ int arb_fused_step(arb_batch* b, const double* dts, int nsteps) {
 // One step in two halves (arb_step_begin / arb_step_end): identity assignment, the caller's
 // state arrays, so that everything the caller reads between the halves is in place.
 int arb_fused_step_half(arb_batch* b, double dt, int half) {
-  int rc = ensure_fused_scratch(b);
+  int rc = half == 0 ? group_refuses_applied(b) : 0;
+  if (rc) return rc;
+  rc = ensure_fused_scratch(b);
   if (rc) return rc;
   FusedState* f = b->fused;
   const int64_t W = b->d.W;
@@ -485,7 +505,7 @@ int arb_fused_step_half(arb_batch* b, double dt, int half) {
     if (grp)
       k_fused_prepare_group<<<(unsigned)((W + GROUP_WPC - 1) / GROUP_WPC), GROUP_WPC * ARB_GL, group_smem_bytes(b), b->stream>>>(b->m, b->d, dt, 1);
     else
-      k_fused_prepare_lane<<<(unsigned)((W + PREP_THREADS - 1) / PREP_THREADS), PREP_THREADS, 0, b->stream>>>(b->m, b->d, dt);
+      launch_prepare_lane(b, b->d, dt);
     if (b->m.nc > 0) launch_gs(b, b->d, dt);
     b->launches += (b->m.nc > 0) ? 2 : 1;
   } else {

@@ -41,6 +41,8 @@ struct arb_batch {
   int half_open = 0;               // arb_step_begin ran the fused stages: arb_step_end must run the finish stage
   int prepare_group = 0;           // 1: prepare stage with 16 lanes per world and on-chip scratch (arb_group.cuh) + K-matrix finish
   int last_fused = 0;              // 1: the constraint read-backs come from the fused scratch (last step was fused)
+  DevApplied applied = {nullptr, nullptr, nullptr};   // arb_batch_bind_applied_forces
+  int* applied_rows = nullptr;     // device [nj]: applied.row (allocated on the first bind)
 };
 
 const char* arb_set_error(const std::string& s);

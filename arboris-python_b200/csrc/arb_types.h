@@ -98,6 +98,15 @@ struct DevModel {
   const int *gvslot;                           // [nj] slot of body j+1's (V, V^) in the forward pass (or -1: never re-read)
 };
 
+// Applied forces of a batch (arb_batch_bind_applied_forces), by WORLD index; nullptr: none.  A kernel
+// argument of their own, given only to the kernels that add them: in DevBatch they change ptxas's
+// register allocation of the Gauss-Seidel kernels, which never read them (more spills, 0.3 % slower).
+struct DevApplied {
+  const double *tau;     // [ndof][W]     generalized forces (caller-owned)
+  const double *wrench;  // [nsel][6][W]  [torque; force] in ground axes at the body origin (caller-owned)
+  const int *row;        // [nj]          wrench row of body j+1, or -1 (library-owned table)
+};
+
 // Per-batch memory: caller-owned state and the phase-API scratch are [elem][W]; the fused
 // scratch (f*, a*) is tiled [W/32][elem][32].
 struct DevBatch {

@@ -248,7 +248,9 @@ ARB_D bool world_invert(double* Y, double* perm, int n, int64_t W, int64_t w) {
   return ok;
 }
 
-ARB_D void world_update_controllers(const DevModel& m, const DevBatch& b, int64_t w, double dt) {
+// ap: the applied forces of arb_batch_bind_applied_forces (none by default)
+ARB_D void world_update_controllers(const DevModel& m, const DevBatch& b, int64_t w, double dt,
+                                    const DevApplied& ap = DevApplied{nullptr, nullptr, nullptr}) {
   const int64_t W = b.W;
   const int n = m.ndof;
   for (int i = 0; i < n; ++i) AT(b.gforce, i) = 0.;
@@ -317,6 +319,29 @@ ARB_D void world_update_controllers(const DevModel& m, const DevBatch& b, int64_
       }
     }
   }
+  // applied forces (arb_batch_bind_applied_forces), a controller registered after the model's with
+  // no impedance: gforce += tau + sum_b J_b^T [R_b^T torque_b; R_b^T force_b]
+  if (ap.tau)
+    for (int k = 0; k < n; ++k) AT(b.gforce, k) += ap.tau[(int64_t)k * W + w];
+  if (ap.wrench)
+    for (int j = 0; j < m.nj; ++j) {
+      const int row = ap.row[j];
+      if (row < 0) continue;
+      Se3 H;
+      load_pose(b, j + 1, w, H);
+      double wg[6], wr[6];
+#pragma unroll
+      for (int i = 0; i < 6; ++i) wg[i] = ap.wrench[(int64_t)(6 * row + i) * W + w];
+      m3t_mulv(H.R, wg, wr);
+      m3t_mulv(H.R, wg + 3, wr + 3);
+      const int off = m.coloff[j + 1], kc = m.kcols[j + 1];
+      for (int l = 0; l < kc; ++l) {
+        double t = 0.;
+#pragma unroll
+        for (int i = 0; i < 6; ++i) t += AT(b.J, (off + l) * 6 + i) * wr[i];
+        AT(b.gforce, m.pathdof[off + l]) += t;
+      }
+    }
   // Y = Z^-1                                                            (core.py:818)
   for (int i = 0; i < n * n; ++i) AT(b.Y, i) = AT(b.Z, i);
   if (!world_invert(b.Y, b.tmp, n, W, w)) b.status[w] |= ARB_STATUS_SINGULAR;

@@ -155,7 +155,8 @@ int arb_batch_set_stream(arb_batch *batch, void *stream);
  *  "prepare_group" 1: the prepare stage runs with a group of 16 lanes per world and the world's
  *                 intermediates in shared memory (csrc/arb_group.cuh), the finish stage as
  *                 q'+ = q_free + K y; same results to 1e-10 (other summation order), 5x slower than the
- *                 default lane-per-world stages on human36 (DESIGN.md 3.4): an A/B switch;
+ *                 default lane-per-world stages on human36 (DESIGN.md 3.4): an A/B switch; it does not
+ *                 support applied forces (arb_batch_bind_applied_forces);
  *  "time_stages"  1: CUDA events around every fused stage, synchronising after every step -- a
  *                 diagnostic for bench.py, read with arb_batch_stage_ms; setting it clears the
  *                 accumulators */
@@ -176,6 +177,24 @@ int arb_batch_bind_controller_params(arb_batch *batch, const double *kp, const d
                                      const double *gpos_des, const double *gvel_des);
 /* dof of each row of those arrays: writes min(npd, cap) entries, returns npd (dofs may be NULL) */
 int arb_model_pd_dofs(const arb_model *model, int32_t *dofs, int cap);
+/* Per-world applied forces: what a reference Controller whose update() returns (gforce, 0) adds,
+ * as one such controller registered AFTER the model's ones, with no impedance term.
+ *  gforce : DEVICE [ndof][W] generalized forces, added to World._gforce (core.py:811-818).
+ *  wrench : DEVICE [nbodies][6][W] wrenches [torque; force] in GROUND axes acting at the origin of
+ *           the frame of body bodies[i]; the step adds J_b^T [R_b^T torque; R_b^T force], with J_b the
+ *           body Jacobian in the body frame (core.py:1171-1176) and R_b the body's rotation at the
+ *           start of the step.
+ *  bodies : HOST list of nbodies distinct body indices 1..njoints (as in arb_get_body; the ground
+ *           is refused), copied into a table of the batch.
+ * Both arrays are caller-owned like the state, world index fastest, and read (by WORLD index,
+ * whatever the thread assignment) at every step of arb_update_controllers, arb_step and
+ * arb_step_begin: write them in place, in stream order, to change the forces between calls.
+ * A NULL pointer or nbodies = 0 means no such force; all NULL / 0 unbinds.  -1 for a body out of
+ * range, the ground, a duplicate body or a wrench without bodies (the previous binding is kept).
+ * The "prepare_group" option does not support them: arb_step / arb_step_begin return -1 while
+ * both are set. */
+int arb_batch_bind_applied_forces(arb_batch *batch, const double *gforce, int nbodies, const int32_t *bodies,
+                                  const double *wrench);
 /* which implementation arb_step runs for this batch: 1 = the fused stages, 0 = the four phase
  * kernels (a PD controller with off-diagonal gains or two controllers on one dof -- Z then has
  * entries the per-dof articulated elimination does not fold -- or the "force_phases" option).
