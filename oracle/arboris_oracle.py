@@ -223,6 +223,47 @@ def joint_djacobian(t, q, dq):
     return dJ
 
 
+def softfinger_solve(v, A, f0, sdist, mu, eps, dt):
+    """SoftFingerContact.solve constraints.py:780-836 for one contact: constraint velocity v (4),
+    admittance block A (4x4), force f0 (4), signed distance, friction mu, eps (3), time step.  Keeps the
+    reference's scalar inner-product quirk: Y_c, beta and b are 1-D, so every dot(x, y.T) below is a
+    scalar that broadcasts over the 3x3 blocks.  Returns (branch, new force, force increment, (B, s) of a
+    sliding solve or None)."""
+    adm, vel, force0 = A, v, np.array(f0, dtype=float)
+    vel_no_force = vel - dot(adm, force0)
+    if sdist + dt*vel_no_force[3] > 0:
+        return BR_SEPARATING, zeros(4), -force0, None
+    dforce = dot(-pinv(adm), hstack((vel[0:3], vel[3] + sdist/dt)))
+    force = force0 + dforce
+    if sum((force[0:3]/eps)**2) <= (force[3]*mu)**2:
+        return BR_STATIC, force, dforce, None
+    alpha = vel - dot(adm, force0)
+    alpha[3] += sdist/dt
+    Y_c = adm[0:3, 3]
+    y_n = adm[3, 3]
+    Y_t = adm[0:3, 0:3]
+    beta = alpha[0:3] - alpha[3]/y_n*Y_c
+    a = mu/y_n*alpha[3]
+    b = mu/y_n*Y_c
+    B = zeros((6, 6))
+    E = diag(eps**2)
+    Y_that = Y_t - dot(Y_c, Y_c.T)/y_n
+    B[3:6, 3:6] = dot(E, Y_that)
+    B[0:3, 0:3] = dot(E, Y_that + 2/a*dot(beta, b.T))
+    B[0:3, 3:6] = -dot(E, dot(beta, beta.T)/(a**2))
+    B[3:6, 0:3] = dot(E, dot(b, b.T)) - eye(3)
+    S = eigvals(B)
+    S = S[np.logical_and(S.imag == 0, S.real <= 0)]
+    if len(S) == 0:
+        s = -1e10
+    else:
+        s = max(min(S.real), -1e10)
+    A2 = adm.copy()
+    A2[0:3, 0:3] -= s*diag(eps**-2)
+    newf = solve(A2, -alpha)
+    return BR_SLIDING, newf, newf - force0, (B.copy(), s)
+
+
 # --------------------------------------------------------------------------
 # the world
 # --------------------------------------------------------------------------
@@ -578,53 +619,15 @@ class OracleWorld(object):
             return df
 
     def _solve_softfinger(self, c, vel, adm, dt, rows):
-        """SoftFingerContact.solve constraints.py:780-836 (with its scalar
-        inner-product quirk: Y_c, beta and b are 1-D, so every dot(x, y.T) below
-        is a scalar that broadcasts over the 3x3 blocks)."""
+        """SoftFingerContact.solve constraints.py:780-836 (softfinger_solve below)."""
         f = self.cforce
         force0 = f[rows].copy()
-        sdist = self.sdist[c]
-        mu = self.cd[c][36]
-        eps = self.cd[c][37:40]
-        vel_no_force = vel - dot(adm, force0)
-        if sdist + dt*vel_no_force[3] > 0:
-            f[rows] = 0.
-            self.branch[c] = BR_SEPARATING
-            return -force0
-        dforce = dot(-pinv(adm), hstack((vel[0:3], vel[3] + sdist/dt)))
-        force = force0 + dforce
-        if sum((force[0:3]/eps)**2) <= (force[3]*mu)**2:
-            f[rows] = force
-            self.branch[c] = BR_STATIC
-            return dforce
-        alpha = vel - dot(adm, force0)
-        alpha[3] += sdist/dt
-        Y_c = adm[0:3, 3]
-        y_n = adm[3, 3]
-        Y_t = adm[0:3, 0:3]
-        beta = alpha[0:3] - alpha[3]/y_n*Y_c
-        a = mu/y_n*alpha[3]
-        b = mu/y_n*Y_c
-        B = zeros((6, 6))
-        E = diag(eps**2)
-        Y_that = Y_t - dot(Y_c, Y_c.T)/y_n
-        B[3:6, 3:6] = dot(E, Y_that)
-        B[0:3, 0:3] = dot(E, Y_that + 2/a*dot(beta, b.T))
-        B[0:3, 3:6] = -dot(E, dot(beta, beta.T)/(a**2))
-        B[3:6, 0:3] = dot(E, dot(b, b.T)) - eye(3)
-        S = eigvals(B)
-        S = S[np.logical_and(S.imag == 0, S.real <= 0)]
-        if len(S) == 0:
-            s = -1e10
-        else:
-            s = max(min(S.real), -1e10)
-        A = adm.copy()
-        A[0:3, 0:3] -= s*diag(eps**-2)
-        newf = solve(A, -alpha)
+        br, newf, df, slide = softfinger_solve(vel, adm, force0, self.sdist[c], self.cd[c][36], self.cd[c][37:40], dt)
         f[rows] = newf
-        self.branch[c] = BR_SLIDING
-        self.last_slide = (B.copy(), s)
-        return newf - force0
+        self.branch[c] = br
+        if slide is not None:
+            self.last_slide = slide
+        return df
 
     # -- integrate  (core.py:974-980) ----------------------------------------------
     def integrate(self, dt):

@@ -219,4 +219,23 @@ void ht_exp(const double* tw, double* out12) {
   se3_exp(tw, h);
   se3_to12(h, out12);
 }
+// SoftFingerContact.solve, phase form: f (4) in/out, df (4) out, *status out; returns the branch
+int ht_softfinger_solve(const double* v, const double* A, const double* P, double sdist, double mu, const double* eps,
+                        double dt, double* f, double* df, int* status) {
+  *status = 0;
+  return softfinger_solve(v, A, P, sdist, mu, eps, dt, f, df, status);
+}
+double ht_inv_cond4(const double* a, double* out) { return inv_small_cond<4>(a, out); }
+int ht_certify(const double* p, double x) { return poly6_certify(p, x) ? 1 : 0; }
+void ht_zaligned(const double* z, double* R, int* idx) { zaligned(z, R, idx); }
+// contact_collide, frames as 12 doubles (R row-major, p); cd: ARB_CONS_NDBL doubles
+double ht_collide(int pair, const double* cd, const double* h0, const double* h1, double* c0, double* c1, int* zi) {
+  Se3 g0, g1, o0, o1;
+  for (int k = 0; k < 9; ++k) { g0.R[k] = h0[k]; g1.R[k] = h1[k]; }
+  for (int k = 0; k < 3; ++k) { g0.p[k] = h0[9 + k]; g1.p[k] = h1[9 + k]; }
+  const double sd = contact_collide(pair, cd, g0, g1, o0, o1, zi);
+  se3_to12(o0, c0);
+  se3_to12(o1, c1);
+  return sd;
+}
 }
