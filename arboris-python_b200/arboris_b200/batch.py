@@ -66,6 +66,8 @@ class BatchedWorld(object):
         self._ctrl_params = {}
         self.applied_gforce = self.applied_wrench = None
         self.applied_bodies = ()
+        self.body_inertia = self.gravity = None
+        self.inertia_bodies = ()
         why = C.c_char_p()
         if self._lib.arb_batch_step_path(self._batch_h, C.byref(why)) == 0:
             # not silent: the fused stages fold controllers per dof; anything else runs the
@@ -155,6 +157,14 @@ class BatchedWorld(object):
         _capi.check(self._lib, self._lib.arb_batch_bind_controller_params(self._batch_h, *ptr))
 
     # ---- per-world applied forces --------------------------------------------------------------
+    def _device_f64(self, v, shape, name):
+        """fp64 contiguous tensor on the batch's device (the argument itself when it already is one)"""
+        t = torch.as_tensor(np.ascontiguousarray(v) if isinstance(v, np.ndarray) else v,
+                            dtype=torch.float64).to(self.device).contiguous()
+        if tuple(t.shape) != shape:
+            raise ValueError("%s must have shape %s, not %s" % (name, shape, tuple(t.shape)))
+        return t
+
     def set_applied_forces(self, gforce=None, wrench=None, bodies=None):
         """Per-world forces of a controller added after the model's ones (what a reference
         ``Controller`` whose ``update`` returns ``(gforce, 0)`` adds):
@@ -166,14 +176,7 @@ class BatchedWorld(object):
         are ``applied_gforce`` and ``applied_wrench`` (the argument itself when it already is one):
         write into them in place to change the forces between steps without another call."""
         W = self.nworlds
-
-        def dev(v, shape, name):
-            t = torch.as_tensor(np.ascontiguousarray(v) if isinstance(v, np.ndarray) else v,
-                                dtype=torch.float64).to(self.device).contiguous()
-            if tuple(t.shape) != shape:
-                raise ValueError("%s must have shape %s, not %s" % (name, shape, tuple(t.shape)))
-            return t
-
+        dev = self._device_f64
         g, wr, bd = self.applied_gforce, self.applied_wrench, self.applied_bodies
         if gforce is False:
             g = None
@@ -196,6 +199,44 @@ class BatchedWorld(object):
             ids, wr.data_ptr() if wr is not None else None))
         self.applied_gforce, self.applied_wrench = g, wr
         self.applied_bodies = bd if wr is not None else ()
+
+    # ---- per-world body inertia and gravity ----------------------------------------------------
+    def set_body_inertia(self, inertia=None, bodies=None):
+        """Per-world inertia of the bodies ``bodies`` (indices as in ``body()``, the ground excluded):
+        ``inertia`` (len(bodies), 10, W), per body and world ``[m, m c_x, m c_y, m c_z, I_xx, I_yy,
+        I_zz, I_xy, I_xz, I_yz]`` (``massmatrix.to_params``), the mass matrix that replaces the
+        model's ``body_mass`` of that body in that world.  Numpy or torch; ``None`` keeps what is bound
+        (``bodies`` too), ``False`` unbinds.  The bound fp64 device tensor is ``body_inertia`` (the
+        argument itself when it already is one): write into it in place to change the inertia between
+        steps without another call."""
+        W = self.nworlds
+        p, bd = self.body_inertia, self.inertia_bodies
+        if inertia is False:
+            p, bd = None, ()
+        else:
+            if bodies is not None:
+                bd = tuple(int(b) for b in np.asarray(bodies).reshape(-1))
+            if inertia is not None:
+                p = self._device_f64(inertia, (len(bd), 10, W), "inertia")
+            elif p is not None and tuple(p.shape) != (len(bd), 10, W):
+                raise ValueError("the bound inertia has %d bodies, not %d: pass the inertia with its bodies"
+                                 % (p.shape[0], len(bd)))
+        ids = (C.c_int32*max(len(bd), 1))(*bd)
+        self._sync_stream()         # (the body table is replaced in stream order)
+        _capi.check(self._lib, self._lib.arb_batch_bind_body_inertia(
+            self._batch_h, len(bd) if p is not None else 0, ids, p.data_ptr() if p is not None else None))
+        self.body_inertia = p
+        self.inertia_bodies = bd if p is not None else ()
+
+    def set_gravity(self, gravity=None):
+        """Per-world gravity ``(3, W)`` in ground axes, in place of ``sum gravity * up`` of the model's
+        WeightControllers (a model without one refuses it).  ``None`` keeps what is bound, ``False``
+        unbinds; the bound fp64 device tensor is ``gravity``, to be written in place between steps."""
+        if gravity is None:
+            return
+        g = None if gravity is False else self._device_f64(gravity, (3, self.nworlds), "gravity")
+        _capi.check(self._lib, self._lib.arb_batch_bind_gravity(self._batch_h, g.data_ptr() if g is not None else None))
+        self.gravity = g
 
     # ---- the four phases and the fused step ---------------------------------------------
     def update_dynamic(self):
@@ -411,7 +452,10 @@ class HostPipeline(object):
     another and the device->host copy of a third overlap (PCIe is full duplex; the step of 262144
     human36 worlds and the two 268 MB copies take about as long).
     ``gpos``, ``gvel``, ``cforce`` are C-contiguous (elem, W) numpy arrays over PINNED memory
-    (e.g. ``torch.empty(...).pin_memory().numpy()``), updated in place."""
+    (e.g. ``torch.empty(...).pin_memory().numpy()``), updated in place.
+    Every block is a batch of its own, so per-world inputs bound on one ``BatchedWorld``
+    (``set_controller_params``, ``set_applied_forces``, ``set_body_inertia``, ``set_gravity``) do not
+    reach the pipeline: it steps the model's parameters."""
 
     def __init__(self, world_or_model, nworlds, chunks="auto", device=None, mode="serial",
                  compute_streams="priority"):

@@ -21,6 +21,7 @@ on the device and copied to the host once, in ``finish()``.
 import numpy as np
 import torch
 
+from . import massmatrix
 from .core import Observer
 from .flatten import JOINT_NDOF, JOINT_NGPOS
 
@@ -154,7 +155,10 @@ class BatchedEnergyMonitor(Observer):
     """Kinetic, potential and mechanical energy of every world at every step
     (``EnergyMonitor``, observers.py:14-54; the attribute names are the reference's).
     The kinetic energy ``gvel^T M gvel / 2`` is evaluated body by body,
-    ``sum_b T_b^T M_b T_b / 2`` with ``T_b = J_b gvel``, so the mass matrix is not assembled."""
+    ``sum_b T_b^T M_b T_b / 2`` with ``T_b = J_b gvel``, so the mass matrix is not assembled.
+    Bodies with per-world inertia (``BatchedWorld.set_body_inertia``) count with each world's own
+    matrix, and with per-world gravity (``set_gravity``) the potential energy is
+    ``-sum_b m_b g_w . p_com,b`` instead of ``9.81 sum_b m_b up . p_com,b``."""
     fused_ok = True
 
     def init(self, world, timeline):
@@ -181,13 +185,35 @@ class BatchedEnergyMonitor(Observer):
         self.time.append(w.current_time)
         Ec = torch.zeros(w.nworlds, dtype=torch.float64, device=w.device)
         Ep = torch.zeros_like(Ec)
-        for k in self._bodies:
-            T = w.body("twist", k + 1)                       # (W, 6)
-            Ec += 0.5*torch.einsum("wi,ij,wj->w", T, self._M[k], T)
-            H = w.body("pose", k + 1)                        # (W, 4, 4)
-            h = torch.einsum("wij,j->wi", H, self._com[k])[:, :3] @ self._up
-            Ep += self._M[k][3, 3]*h
-        Ep *= 9.81
+        bound = getattr(w, "inertia_bodies", ())
+        g = getattr(w, "gravity", None)
+        if not bound and g is None:
+            for k in self._bodies:
+                T = w.body("twist", k + 1)                       # (W, 6)
+                Ec += 0.5*torch.einsum("wi,ij,wj->w", T, self._M[k], T)
+                H = w.body("pose", k + 1)                        # (W, 4, 4)
+                h = torch.einsum("wij,j->wi", H, self._com[k])[:, :3] @ self._up
+                Ep += self._M[k][3, 3]*h
+            Ep *= 9.81
+        else:
+            for k in sorted(set(self._bodies) | {b - 1 for b in bound}):
+                if k + 1 in bound:                               # (W, 6, 6): the world's own M_b
+                    M = massmatrix.from_params(w.body_inertia[bound.index(k + 1)].T)
+                    m = M[:, 3, 3]
+                    com = torch.stack((M[:, 2, 4], M[:, 0, 5], M[:, 1, 3]), 1)
+                    com = torch.where((m > 0)[:, None], com/torch.where(m > 0, m, 1.)[:, None], 0.)
+                    com = torch.cat((com, torch.ones_like(m)[:, None]), 1)
+                else:
+                    M = self._M[k].expand(w.nworlds, 6, 6)
+                    m = M[:, 3, 3]
+                    com = self._com[k].expand(w.nworlds, 4)
+                T = w.body("twist", k + 1)
+                Ec += 0.5*torch.einsum("wi,wij,wj->w", T, M, T)
+                p = torch.einsum("wij,wj->wi", w.body("pose", k + 1), com)[:, :3]
+                if g is None:
+                    Ep += 9.81*m*(p @ self._up)
+                else:
+                    Ep -= m*(p*g.T).sum(1)
         self.kinetic_energy.append(Ec)
         self.potential_energy.append(Ep)
         self.mechanichal_energy.append(Ec + Ep)

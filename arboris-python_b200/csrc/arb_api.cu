@@ -163,6 +163,7 @@ extern "C" void arb_batch_destroy(arb_batch* b) {
   cudaFree(b->scratch_int);
   cudaFree(b->d.status);
   cudaFree(b->applied_rows);
+  cudaFree(b->inertia_rows);
   arb_fused_release(b);
   delete b;
 }
@@ -235,6 +236,34 @@ extern "C" int arb_batch_bind_applied_forces(arb_batch* b, const double* gforce,
   return 0;
 }
 
+extern "C" int arb_batch_bind_body_inertia(arb_batch* b, int nbodies, const int32_t* bodies, const double* inertia) {
+  if (!b) { arb_set_error("null batch"); return -1; }
+  std::vector<int> rows;
+  std::string err;
+  if (applied_wrench_rows(b->model->host, nbodies, bodies, inertia != nullptr, rows, err, "inertia")) {
+    arb_set_error(err);
+    return -1;
+  }
+  CUDA_OK(cudaSetDevice(b->device));
+  if (!b->inertia_rows) CUDA_OK(cudaMalloc((void**)&b->inertia_rows, sizeof(int) * rows.size()));
+  // in stream order: the steps already enqueued read the previous table
+  CUDA_OK(cudaMemcpyAsync(b->inertia_rows, rows.data(), sizeof(int) * rows.size(), cudaMemcpyHostToDevice, b->stream));
+  CUDA_OK(cudaStreamSynchronize(b->stream));
+  b->applied.inertia = nbodies > 0 ? inertia : nullptr;
+  b->applied.irow = b->inertia_rows;
+  return 0;
+}
+
+extern "C" int arb_batch_bind_gravity(arb_batch* b, const double* gravity) {
+  if (!b) { arb_set_error("null batch"); return -1; }
+  if (gravity && b->model->host.nweight == 0) {
+    arb_set_error("the model has no WeightController: there is no gravity to replace");
+    return -1;
+  }
+  b->applied.gravity = gravity;
+  return 0;
+}
+
 /* 1: arb_step runs the fused stages; 0: it runs the four phase kernels (a controller couples dofs
  * in a way the fused stages do not fold, or "force_phases" is set); *why (optional) names the reason */
 extern "C" int arb_batch_step_path(const arb_batch* b, const char** why) {
@@ -255,13 +284,17 @@ static int check_bound(arb_batch* b) {
 // ---------------------------------------------------------------------------------
 #define LPW_THREADS 64
 
-__global__ void __launch_bounds__(LPW_THREADS) k_update_dynamic(DevModel m, DevBatch b) {
+// PARAMS: the instantiations with the world's body inertia and gravity, launched only while either
+// is bound (arb_batch_bind_body_inertia / _gravity)
+template <bool PARAMS>
+__global__ void __launch_bounds__(LPW_THREADS) k_update_dynamic(DevModel m, DevBatch b, DevApplied ap) {
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (w < b.W) world_update_dynamic(m, b, w);
+  if (w < b.W) world_update_dynamic<PARAMS>(m, b, w, ap);
 }
+template <bool PARAMS>
 __global__ void __launch_bounds__(LPW_THREADS) k_update_controllers(DevModel m, DevBatch b, double dt, DevApplied ap) {
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (w < b.W) world_update_controllers(m, b, w, dt, ap);
+  if (w < b.W) world_update_controllers<PARAMS>(m, b, w, dt, ap);
 }
 __global__ void __launch_bounds__(LPW_THREADS) k_update_constraints(DevModel m, DevBatch b, double dt) {
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -273,6 +306,16 @@ __global__ void __launch_bounds__(LPW_THREADS) k_integrate(DevModel m, DevBatch 
 }
 
 static inline unsigned lpw_grid(int64_t W) { return (unsigned)((W + LPW_THREADS - 1) / LPW_THREADS); }
+static inline bool params_bound(const arb_batch* b) { return b->applied.inertia || b->applied.gravity; }
+static void launch_update_dynamic(arb_batch* b) {
+  if (params_bound(b)) k_update_dynamic<true><<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, b->applied);
+  else k_update_dynamic<false><<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, b->applied);
+}
+static void launch_update_controllers(arb_batch* b, double dt) {
+  if (params_bound(b))
+    k_update_controllers<true><<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->applied);
+  else k_update_controllers<false><<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->applied);
+}
 
 #define LAUNCH_CHECK(b)                                                        \
   do {                                                                         \
@@ -288,7 +331,7 @@ extern "C" int arb_update_dynamic(arb_batch* b) {
   int rc = check_bound(b); if (rc) return rc;
   CUDA_OK(cudaSetDevice(b->device));
   rc = arb_ensure_phase_scratch(b); if (rc) return rc;
-  k_update_dynamic<<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d);
+  launch_update_dynamic(b);
   LAUNCH_CHECK(b);
   b->last_fused = 0;
   b->half_open = 0;
@@ -299,7 +342,7 @@ extern "C" int arb_update_controllers(arb_batch* b, double dt) {
   if (!(dt > 0)) { arb_set_error("dt must be > 0"); return -3; }
   CUDA_OK(cudaSetDevice(b->device));
   rc = arb_ensure_phase_scratch(b); if (rc) return rc;
-  k_update_controllers<<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->applied);
+  launch_update_controllers(b, dt);
   LAUNCH_CHECK(b);
   return 0;
 }
@@ -331,8 +374,8 @@ int arb_step_phases(arb_batch* b, const double* dts, int nsteps) {
   for (int s = 0; s < nsteps; ++s) {
     const double dt = dts[s];
     if (!(dt > 0)) { arb_set_error("dt must be > 0"); return -3; }
-    k_update_dynamic<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d);
-    k_update_controllers<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->applied);
+    launch_update_dynamic(b);
+    launch_update_controllers(b, dt);
     k_update_constraints<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt);
     k_integrate<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt);
     b->launches += 3;
@@ -477,7 +520,7 @@ __global__ void k_gather_tiled(const T* __restrict__ src, T* __restrict__ out, i
   const int64_t ww = slots ? (int64_t)slots[w0 + w] : w0 + w;   // the scratch belongs to the thread slot
   out[i] = src[(ww / ARB_TILE) * rec * ARB_TILE + (int64_t)e * stride * ARB_TILE + ww % ARB_TILE];
 }
-__global__ void k_get_body(DevModel m, DevBatch b, int which, int body, double* out, int64_t w0, int64_t nw) {
+__global__ void k_get_body(DevModel m, DevBatch b, DevApplied ap, int which, int body, double* out, int64_t w0, int64_t nw) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= nw) return;
   const int64_t w = w0 + i, W = b.W;
@@ -510,15 +553,17 @@ __global__ void k_get_body(DevModel m, DevBatch b, int which, int body, double* 
     for (int r = 0; r < 36; ++r) { Om[r] = 0.; o[r] = 0.; }
     if (body == 0) return;
     skew3(t, wx);
-    m3_mul(m.brx + 9 * (body - 1), wx, t1);
-    m3_mul(wx, m.brx + 9 * (body - 1), t2);
+    const double *Mb, *rx;
+    double Mw[36], rxw[9];
+    world_body_mass<true>(m, ap, body - 1, W, w, Mb, rx, Mw, rxw);   // the world's own M_b if bound
+    m3_mul(rx, wx, t1);
+    m3_mul(wx, rx, t2);
     for (int r = 0; r < 3; ++r)
       for (int c = 0; c < 3; ++c) {
         Om[6 * r + c] = wx[3 * r + c];
         Om[6 * (r + 3) + c + 3] = wx[3 * r + c];
         Om[6 * r + c + 3] = t1[3 * r + c] - t2[3 * r + c];
       }
-    const double* Mb = m.bmass + 36 * (body - 1);
     for (int r = 0; r < 6; ++r)
       for (int c = 0; c < 6; ++c) {
         double s = 0.;
@@ -603,7 +648,7 @@ extern "C" int arb_get_body(arb_batch* b, int which, int body, double* out, int6
     LAUNCH_CHECK(b);
     return 0;
   }
-  k_get_body<<<(unsigned)((nw + 127) / 128), 128, 0, b->stream>>>(b->m, b->d, which, body, out, w0, nw);
+  k_get_body<<<(unsigned)((nw + 127) / 128), 128, 0, b->stream>>>(b->m, b->d, b->applied, which, body, out, w0, nw);
   LAUNCH_CHECK(b);
   return 0;
 }

@@ -323,14 +323,22 @@ ARB_D double artic_pd_diag(const DevModel& m, const DevBatch& b, int64_t w, int 
 // reduced right-hand side u of the free motion (w_b = M_b (T_b/dt + gravity_b) + applied wrench,
 // tau = PD + applied generalized force).  APPLIED = false: the instantiation without the applied-force
 // terms, which the fused step runs while none are bound (with them ptxas spills 48 more bytes in the
-// prepare kernel, a cost the unbound step need not pay).
-template <bool APPLIED>
+// prepare kernel, a cost the unbound step need not pay).  PARAMS = true (with APPLIED): M_b, rx and the
+// body flags of the bodies in ap.irow, and gravity, are the world's own (arb_batch_bind_body_inertia,
+// arb_batch_bind_gravity); the instantiation the step runs while either is bound.
+template <bool APPLIED, bool PARAMS = false>
 ARB_D bool artic_factor(const DevModel& m, const DevBatch& b, int64_t w, double dt, const DevApplied& ap) {
   bool ok = true;
   // 1/dt once per world: the 36 M_b/dt per body are mostly 0/dt, which sends the fp64 division
   // through its slow path (a quarter of this stage's instructions before)
   const double idt = 1. / dt;
-  const double gt[6] = {0., 0., 0., m.gravity * m.up[0], m.gravity * m.up[1], m.gravity * m.up[2]};
+  double gt[6] = {0., 0., 0., m.gravity * m.up[0], m.gravity * m.up[1], m.gravity * m.up[2]};
+  if constexpr (PARAMS) {
+    if (ap.gravity) {
+#pragma unroll
+      for (int i = 0; i < 3; ++i) gt[3 + i] = arb_ld_state(ap.gravity + (int64_t)i * b.W + artic_param_world(b, w));
+    }
+  }
   // Along a chain (joint j+1 hangs on the body of joint j, the usual case in depth-first order) the
   // child's contribution X^T IA X, X^T IM X, X^T beta stays in registers for the next iteration
   // instead of going through its scratch slot: `carry`.
@@ -348,8 +356,27 @@ ARB_D bool artic_factor(const DevModel& m, const DevBatch& b, int64_t w, double 
     const int par = m.jparent[j];
     const int nd = arb_joint_ndof(type);
     const int dof = m.jdof[j];
-    const int flags = m.bflags[j];
+    int flags = m.bflags[j];
     const double* Mb = m.bmass + 36 * j;
+    const double* rx = m.brx + 9 * j;
+    double Mw[36], rxw[9];      // (PARAMS) the world's M_b and rx, in registers
+    if constexpr (PARAMS) {
+      const int row = ap.inertia ? ap.irow[j] : -1;
+      if (row >= 0) {
+        const double* pp = ap.inertia + (int64_t)(10 * row) * b.W + artic_param_world(b, w);
+        double v[10];
+#pragma unroll
+        for (int i = 0; i < 10; ++i) v[i] = arb_ld_state(pp + (int64_t)i * b.W);
+        flags = (flags & ARB_BODY_HASVISC) | body_inertia_matrix(v, Mw, rxw);
+      } else {
+#pragma unroll
+        for (int i = 0; i < 36; ++i) Mw[i] = Mb[i];
+#pragma unroll
+        for (int i = 0; i < 9; ++i) rxw[i] = rx[i];
+      }
+      Mb = Mw;
+      rx = rxw;
+    }
     if (!carry) {
 #pragma unroll
       for (int i = 0; i < 36; ++i) { IA[i] = 0.; IM[i] = 0.; }
@@ -365,8 +392,8 @@ ARB_D bool artic_factor(const DevModel& m, const DevBatch& b, int64_t w, double 
       {
         double wx[9], t1[9], t2[9];
         skew3(T, wx);
-        m3_mul(m.brx + 9 * j, wx, t1);
-        m3_mul(wx, m.brx + 9 * j, t2);
+        m3_mul(rx, wx, t1);
+        m3_mul(wx, rx, t2);
 #pragma unroll
         for (int i = 0; i < 9; ++i) X3[i] = t1[i] - t2[i];
       }

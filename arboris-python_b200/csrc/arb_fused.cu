@@ -81,18 +81,21 @@ struct FusedState {
 #ifndef FINISH_THREADS
 #define FINISH_THREADS 128
 #endif
-template <bool APPLIED>
+template <bool APPLIED, bool PARAMS>
 __global__ void __launch_bounds__(PREP_THREADS, PREP_MINBLOCKS) k_fused_prepare_lane(DevModel m, DevBatch b, double dt, DevApplied ap) {
   FUSED_SLOT_WORLD();
   if (s >= b.W) return;
-  world_fused_prepare<APPLIED>(m, fused_tile_view(b, s), w, dt, ap);
+  world_fused_prepare<APPLIED, PARAMS>(m, fused_tile_view(b, s), w, dt, ap);
 }
-// the instantiation with the applied-force terms only while some are bound
+// the instantiation with the applied-force terms only while some are bound, and the one that also
+// reads the world's body inertia and gravity only while either is bound
 static void launch_prepare_lane(const arb_batch* b, const DevBatch& d, double dt) {
   const unsigned grid = (unsigned)((d.W + PREP_THREADS - 1) / PREP_THREADS);
-  if (b->applied.tau || b->applied.wrench)
-    k_fused_prepare_lane<true><<<grid, PREP_THREADS, 0, b->stream>>>(b->m, d, dt, b->applied);
-  else k_fused_prepare_lane<false><<<grid, PREP_THREADS, 0, b->stream>>>(b->m, d, dt, b->applied);
+  if (b->applied.inertia || b->applied.gravity)
+    k_fused_prepare_lane<true, true><<<grid, PREP_THREADS, 0, b->stream>>>(b->m, d, dt, b->applied);
+  else if (b->applied.tau || b->applied.wrench)
+    k_fused_prepare_lane<true, false><<<grid, PREP_THREADS, 0, b->stream>>>(b->m, d, dt, b->applied);
+  else k_fused_prepare_lane<false, false><<<grid, PREP_THREADS, 0, b->stream>>>(b->m, d, dt, b->applied);
 }
 // Threads per CTA of the Gauss-Seidel kernel: 128 (8.87 ms against 9.01 with 64 and 9.11 with 32 at
 // 262144 worlds; end to end, with seven column blocks on three streams, 1.406e7 world-steps/s against
@@ -215,12 +218,21 @@ __global__ void __launch_bounds__(FUSED_THREADS) k_fused_finish_k(DevModel m, De
 static size_t group_smem_bytes(const arb_batch* b) { return sizeof(double) * (size_t)b->m.gl.total * GROUP_WPC; }
 // the group stage needs its per-world record to fit the SM's shared memory
 static bool group_supported(const arb_batch* b) { return group_smem_bytes(b) <= 227 * 1024; }
-// the group prepare stage has no applied-force term: refused rather than stepping without the forces
+// the group prepare stage has no applied-force term and reads the model's inertia and gravity:
+// refused rather than stepping without the per-world inputs
 static int group_refuses_applied(const arb_batch* b) {
-  if (!(b->prepare_group && group_supported(b) && (b->applied.tau || b->applied.wrench))) return 0;
-  arb_set_error("the prepare_group option does not support applied forces (arb_batch_bind_applied_forces): "
-                "unbind them or clear the option");
-  return -1;
+  if (!(b->prepare_group && group_supported(b))) return 0;
+  if (b->applied.tau || b->applied.wrench) {
+    arb_set_error("the prepare_group option does not support applied forces (arb_batch_bind_applied_forces): "
+                  "unbind them or clear the option");
+    return -1;
+  }
+  if (b->applied.inertia || b->applied.gravity) {
+    arb_set_error("the prepare_group option does not support per-world body inertia or gravity "
+                  "(arb_batch_bind_body_inertia, arb_batch_bind_gravity): unbind them or clear the option");
+    return -1;
+  }
+  return 0;
 }
 
 // private by-slot state <- caller's state (GATHER) or the reverse; one thread per slot and
@@ -314,8 +326,9 @@ static int ensure_fused_scratch(arb_batch* b) {
     }
     b->gs_plain = plain ? 1 : 0;
   }
-  CUDA_OKF(cudaFuncSetAttribute(k_fused_prepare_lane<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
-  CUDA_OKF(cudaFuncSetAttribute(k_fused_prepare_lane<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_prepare_lane<false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_prepare_lane<true, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_prepare_lane<true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
   CUDA_OKF(cudaFuncSetAttribute(k_fused_finish, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
   b->fused = f;
   return 0;

@@ -135,13 +135,14 @@ ARB_D void fused_gen_rows(const DevModel& m, const DevBatch& b, int64_t w, const
 
 // ---------------------------------------------------------------------------------------
 // prepare: see the header.  Reads the bound state only; writes the fused scratch.
-// APPLIED: with the applied-force terms (arb_batch_bind_applied_forces; artic_factor).
-template <bool APPLIED = false>
+// APPLIED: with the applied-force terms (arb_batch_bind_applied_forces; artic_factor); PARAMS (with
+// APPLIED): with the world's body inertia and gravity (arb_batch_bind_body_inertia / _gravity).
+template <bool APPLIED = false, bool PARAMS = false>
 ARB_D void world_fused_prepare(const DevModel& m, const DevBatch& b, int64_t w, double dt,
                                const DevApplied& ap = DevApplied{nullptr, nullptr, nullptr}) {
   const int NG = m.ngrows;
   artic_kinematics(m, b, w);
-  if (!artic_factor<APPLIED>(m, b, w, dt, ap)) b.status[w] |= ARB_STATUS_SINGULAR;
+  if (!artic_factor<APPLIED, PARAMS>(m, b, w, dt, ap)) b.status[w] |= ARB_STATUS_SINGULAR;
   // frames of the contact-aligned generator bodies: R_e = R_c^T R_body
   for (int gi = 0; gi < m.ngen; ++gi) {
     if (!m.gen_aligned[gi]) continue;

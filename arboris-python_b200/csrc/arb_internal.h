@@ -43,6 +43,7 @@ struct arb_batch {
   int last_fused = 0;              // 1: the constraint read-backs come from the fused scratch (last step was fused)
   DevApplied applied = {nullptr, nullptr, nullptr};   // arb_batch_bind_applied_forces
   int* applied_rows = nullptr;     // device [nj]: applied.row (allocated on the first bind)
+  int* inertia_rows = nullptr;     // device [nj]: applied.irow (arb_batch_bind_body_inertia, allocated on the first bind)
 };
 
 const char* arb_set_error(const std::string& s);

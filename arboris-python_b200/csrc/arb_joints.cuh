@@ -110,3 +110,32 @@ ARB_D void joint_kinematics(int type, const double* q, const double* dq, JointKi
     k.T[r] = t;
   }
 }
+
+// ---------------------------------------------------------------------------------------
+// Per-world inertia of one body (arb_batch_bind_body_inertia): the 10 numbers
+// v = [m, m c_x, m c_y, m c_z, I_xx, I_yy, I_zz, I_xy, I_xz, I_yz] placed into the body's 6x6 mass
+// matrix ([angular; linear], row-major), M = [[I, skew(m c)], [skew(m c)^T, m 1]], without
+// arithmetic; rx = M[0:3,3:6]/M[3,3] or 0 (core.py:1280-1283).  Returns the MASSIVE / HASMASS flags
+// by the rules build_host_model (arb_model_host.h) applies to the model's matrices.
+ARB_D int body_inertia_matrix(const double* v, double* M, double* rx) {
+  const double m = v[0], cx = v[1], cy = v[2], cz = v[3];
+  const double Mv[36] = {v[4], v[7], v[8], 0., -cz, cy,
+                         v[7], v[5], v[9], cz, 0., -cx,
+                         v[8], v[9], v[6], -cy, cx, 0.,
+                         0., cz, -cy, m, 0., 0.,
+                         -cz, 0., cx, 0., m, 0.,
+                         cy, -cx, 0., 0., 0., m};
+  int fl = 0;
+#pragma unroll
+  for (int i = 0; i < 36; ++i) {
+    M[i] = Mv[i];
+    if (Mv[i] > 0.) fl |= ARB_BODY_MASSIVE;
+    if (Mv[i] != 0.) fl |= ARB_BODY_HASMASS;
+  }
+  const bool light = m <= 1e-10;    // (core.py:1280)
+#pragma unroll
+  for (int r = 0; r < 3; ++r)
+#pragma unroll
+    for (int c = 0; c < 3; ++c) rx[3 * r + c] = light ? 0. : Mv[6 * r + 3 + c] / m;
+  return fl;
+}

@@ -420,18 +420,23 @@ static inline void carve_fused(const FusedSizes& s, double* dbl, int* ints, DevB
   b.firec = s.total_ints();
 }
 // Body -> wrench row table of arb_batch_bind_applied_forces: rows[j] = i if bodies[i] == j + 1,
-// else -1.  Refuses the ground, bodies out of range, duplicates and a wrench without bodies.
+// else -1.  Refuses the ground, bodies out of range, duplicates and a wrench without bodies.  The same
+// table for the body inertia of arb_batch_bind_body_inertia, with `what` naming the array.
 static inline int applied_wrench_rows(const HostModel& m, int nbodies, const int32_t* bodies, bool has_wrench,
-                                      std::vector<int>& rows, std::string& err) {
-  if (nbodies < 0) { err = "negative number of wrench bodies"; return -1; }
+                                      std::vector<int>& rows, std::string& err, const char* what = "wrench") {
+  const std::string w(what);
+  if (nbodies < 0) { err = "negative number of " + w + " bodies"; return -1; }
   if (nbodies > 0 && !bodies) { err = "null body list"; return -1; }
-  if (has_wrench && nbodies == 0) { err = "a wrench array needs its bodies"; return -1; }
+  if (has_wrench && nbodies == 0) {
+    err = (std::string("aeiou").find(w[0]) != std::string::npos ? "an " : "a ") + w + " array needs its bodies";
+    return -1;
+  }
   rows.assign(m.nj > 0 ? m.nj : 1, -1);
   for (int i = 0; i < nbodies; ++i) {
     const int body = bodies[i];
-    if (body == 0) { err = "no wrench can be applied to the ground (body 0)"; return -1; }
-    if (body < 0 || body > m.nj) { err = "wrench body " + std::to_string(body) + " out of range"; return -1; }
-    if (rows[body - 1] >= 0) { err = "wrench body " + std::to_string(body) + " listed twice"; return -1; }
+    if (body == 0) { err = "no " + w + " can be applied to the ground (body 0)"; return -1; }
+    if (body < 0 || body > m.nj) { err = w + " body " + std::to_string(body) + " out of range"; return -1; }
+    if (rows[body - 1] >= 0) { err = w + " body " + std::to_string(body) + " listed twice"; return -1; }
     rows[body - 1] = i;
   }
   return 0;

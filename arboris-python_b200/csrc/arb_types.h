@@ -98,13 +98,18 @@ struct DevModel {
   const int *gvslot;                           // [nj] slot of body j+1's (V, V^) in the forward pass (or -1: never re-read)
 };
 
-// Applied forces of a batch (arb_batch_bind_applied_forces), by WORLD index; nullptr: none.  A kernel
-// argument of their own, given only to the kernels that add them: in DevBatch they change ptxas's
-// register allocation of the Gauss-Seidel kernels, which never read them (more spills, 0.3 % slower).
+// Per-world inputs of the free motion, by WORLD index; nullptr: none.  Applied forces
+// (arb_batch_bind_applied_forces), body inertia (arb_batch_bind_body_inertia) and gravity
+// (arb_batch_bind_gravity).  A kernel argument of their own, given only to the kernels that read
+// them: in DevBatch they change ptxas's register allocation of the Gauss-Seidel kernels, which never
+// read them (more spills, 0.3 % slower).
 struct DevApplied {
   const double *tau;     // [ndof][W]     generalized forces (caller-owned)
   const double *wrench;  // [nsel][6][W]  [torque; force] in ground axes at the body origin (caller-owned)
   const int *row;        // [nj]          wrench row of body j+1, or -1 (library-owned table)
+  const double *inertia; // [nsel][10][W] [m, m c, I_xx, I_yy, I_zz, I_xy, I_xz, I_yz] (caller-owned)
+  const int *irow;       // [nj]          inertia row of body j+1, or -1 (library-owned table)
+  const double *gravity; // [3][W]        gravity in ground axes, in place of sum_a gravity_a up (caller-owned)
 };
 
 // Per-batch memory: caller-owned state and the phase-API scratch are [elem][W]; the fused

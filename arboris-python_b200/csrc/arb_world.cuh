@@ -33,8 +33,33 @@ ARB_D void load_twist(const DevBatch& b, int body, int64_t w, double* t) {
   for (int i = 0; i < 6; ++i) t[i] = (body == 0) ? 0. : AT(b.twist, (body - 1) * 6 + i);
 }
 
+// The world's own M_b, rx and body flags of body j+1 (arb_batch_bind_body_inertia) when PARAMS and the
+// body is bound; the model's otherwise.  Mw, rxw: storage for the world's values.
+template <bool PARAMS>
+ARB_D int world_body_mass(const DevModel& m, const DevApplied& ap, int j, int64_t W, int64_t w,
+                          const double*& Mb, const double*& rx, double* Mw, double* rxw) {
+  Mb = m.bmass + 36 * j;
+  rx = m.brx + 9 * j;
+  int flags = m.bflags[j];
+  if constexpr (PARAMS) {
+    const int row = ap.inertia ? ap.irow[j] : -1;
+    if (row >= 0) {
+      double v[10];
+#pragma unroll
+      for (int i = 0; i < 10; ++i) v[i] = ap.inertia[(int64_t)(10 * row + i) * W + w];
+      flags = (flags & ARB_BODY_HASVISC) | body_inertia_matrix(v, Mw, rxw);
+      Mb = Mw;
+      rx = rxw;
+    }
+  }
+  return flags;
+}
+
 // ---------------------------------------------------------------------------
-ARB_D void world_update_dynamic(const DevModel& m, const DevBatch& b, int64_t w) {
+// PARAMS: with the world's body inertia (arb_batch_bind_body_inertia, ap.inertia)
+template <bool PARAMS = false>
+ARB_D void world_update_dynamic(const DevModel& m, const DevBatch& b, int64_t w,
+                                const DevApplied& ap = DevApplied{nullptr, nullptr, nullptr}) {
   const int64_t W = b.W;
   const int n = m.ndof;
   for (int i = 0; i < n * n; ++i) {
@@ -147,16 +172,17 @@ ARB_D void world_update_dynamic(const DevModel& m, const DevBatch& b, int64_t w)
     }
     // M += J^T M_b J ; B += J^T B_b J ; N += J^T (M_b dJ + N_b J)          (core.py:725-734)
     // with N_b = [[w^, rx w^ - w^ rx],[0, w^]] M_b                        (core.py:1276-1288)
-    const int flags = m.bflags[j];
+    const double *Mb, *rx;
+    double Mw[36], rxw[9];
+    const int flags = world_body_mass<PARAMS>(m, ap, j, W, w, Mb, rx, Mw, rxw);
     if (flags & (ARB_BODY_HASMASS | ARB_BODY_HASVISC)) {
-      const double* Mb = m.bmass + 36 * j;
       const double* Bb = m.bvisc + 36 * j;
       double wx[9], X[9];
       {
         double t1[9], t2[9];
         skew3(Tc, wx);
-        m3_mul(m.brx + 9 * j, wx, t1);
-        m3_mul(wx, m.brx + 9 * j, t2);
+        m3_mul(rx, wx, t1);
+        m3_mul(wx, rx, t2);
 #pragma unroll
         for (int i = 0; i < 9; ++i) X[i] = t1[i] - t2[i];
       }
@@ -248,7 +274,9 @@ ARB_D bool world_invert(double* Y, double* perm, int n, int64_t W, int64_t w) {
   return ok;
 }
 
-// ap: the applied forces of arb_batch_bind_applied_forces (none by default)
+// ap: the applied forces of arb_batch_bind_applied_forces (none by default); PARAMS: with the world's
+// body inertia and gravity (ap.inertia, ap.gravity)
+template <bool PARAMS = false>
 ARB_D void world_update_controllers(const DevModel& m, const DevBatch& b, int64_t w, double dt,
                                     const DevApplied& ap = DevApplied{nullptr, nullptr, nullptr}) {
   const int64_t W = b.W;
@@ -256,18 +284,28 @@ ARB_D void world_update_controllers(const DevModel& m, const DevBatch& b, int64_
   for (int i = 0; i < n; ++i) AT(b.gforce, i) = 0.;
   // Z = M/dt + B + N                                                   (core.py:813)
   for (int i = 0; i < n * n; ++i) AT(b.Z, i) = AT(b.M, i) / dt + AT(b.B, i) + AT(b.N, i);
+  bool weighed = false;     // (PARAMS) the world's gravity is evaluated once, at the first WeightController
   for (int a = 0; a < m.na; ++a) {
     if (m.atype[a] == ARB_CTRL_WEIGHT) {
       // gforce += J_b^T M_b Ad(pose_b^-1) [0,0,0, g up]                  (controllers.py:43-60)
       const double grav = m.adbl[4 * a];
       double gt[6] = {0., 0., 0., grav * m.up[0], grav * m.up[1], grav * m.up[2]};
+      if constexpr (PARAMS) {
+        if (ap.gravity) {
+          if (weighed) continue;
+          weighed = true;
+#pragma unroll
+          for (int i = 0; i < 3; ++i) gt[3 + i] = ap.gravity[(int64_t)i * W + w];
+        }
+      }
       for (int j = 0; j < m.nj; ++j) {
-        if (!(m.bflags[j] & ARB_BODY_MASSIVE)) continue;
+        const double *Mb, *rx;
+        double Mw[36], rxw[9];
+        if (!(world_body_mass<PARAMS>(m, ap, j, W, w, Mb, rx, Mw, rxw) & ARB_BODY_MASSIVE)) continue;
         Se3 H;
         load_pose(b, j + 1, w, H);
         double g[6], wr[6];
         iad_apply(H, gt, g);
-        const double* Mb = m.bmass + 36 * j;
 #pragma unroll
         for (int r = 0; r < 6; ++r) {
           double t = 0.;

@@ -156,7 +156,8 @@ int arb_batch_set_stream(arb_batch *batch, void *stream);
  *                 intermediates in shared memory (csrc/arb_group.cuh), the finish stage as
  *                 q'+ = q_free + K y; same results to 1e-10 (other summation order), 5x slower than the
  *                 default lane-per-world stages on human36 (DESIGN.md 3.4): an A/B switch; it does not
- *                 support applied forces (arb_batch_bind_applied_forces);
+ *                 support applied forces (arb_batch_bind_applied_forces), per-world body inertia
+ *                 or gravity (arb_batch_bind_body_inertia, arb_batch_bind_gravity);
  *  "time_stages"  1: CUDA events around every fused stage, synchronising after every step -- a
  *                 diagnostic for bench.py, read with arb_batch_stage_ms; setting it clears the
  *                 accumulators */
@@ -195,6 +196,30 @@ int arb_model_pd_dofs(const arb_model *model, int32_t *dofs, int cap);
  * both are set. */
 int arb_batch_bind_applied_forces(arb_batch *batch, const double *gforce, int nbodies, const int32_t *bodies,
                                   const double *wrench);
+/* Per-world body inertia: the reference keeps one Body.mass per body (a 6x6 matrix in
+ * the body frame, [angular; linear]); a batch may give bodies of every world their own.
+ *  inertia : DEVICE [nbodies][10][W], p = [m, m c_x, m c_y, m c_z, I_xx, I_yy, I_zz, I_xy, I_xz, I_yz]
+ *            per body and world: the independent entries of M_b = [[I, skew(m c)], [skew(m c)^T, m 1]],
+ *            I = [[I_xx, I_xy, I_xz], [I_xy, I_yy, I_yz], [I_xz, I_yz, I_zz]], which replaces the model's
+ *            mass matrix of body bodies[i] in that world.  rx = M[0:3,3:6]/M[3,3] or 0 (core.py:1280),
+ *            whether gravity acts on the body (some entry > 0, controllers.py:35-41) and whether it has
+ *            mass at all are derived per world by the reference's rules.  The values are not checked: a
+ *            world whose impedance they make singular gets ARB_STATUS_SINGULAR (LinAlgError in the
+ *            reference, core.py:818), a NaN ARB_STATUS_NONFINITE in that world only.
+ *  bodies  : HOST list of nbodies distinct body indices 1..njoints, copied into a table of the batch.
+ * NULL or nbodies = 0 unbinds; -1 for a body out of range, the ground, a duplicate body or inertia
+ * without bodies (the previous binding is kept). */
+int arb_batch_bind_body_inertia(arb_batch *batch, int nbodies, const int32_t *bodies, const double *inertia);
+/* Per-world gravity: DEVICE [3][W], the gravity vector of each world in GROUND axes, in place of
+ * sum_a gravity_a * up of the model's WeightControllers (controllers.py:43-60).
+ * NULL unbinds; -1 for a model without a WeightController (there is no gravity to replace).
+ * Both arrays are caller-owned like the state, world index fastest, and read (by WORLD index, whatever
+ * the thread assignment) at every step of arb_update_dynamic, arb_update_controllers, arb_step (fused
+ * stages and phase kernels), arb_step_begin and the host-buffer steps: write them in place, in stream
+ * order, to change them between calls.  arb_get_body(ARB_BODY_NLE) reads the bound inertia too.  The
+ * "prepare_group" option does not support them: arb_step / arb_step_begin return -1 while both are
+ * set. */
+int arb_batch_bind_gravity(arb_batch *batch, const double *gravity);
 /* which implementation arb_step runs for this batch: 1 = the fused stages, 0 = the four phase
  * kernels (a PD controller with off-diagonal gains or two controllers on one dof -- Z then has
  * entries the per-dof articulated elimination does not fold -- or the "force_phases" option).
