@@ -68,6 +68,8 @@ class BatchedWorld(object):
         self.applied_bodies = ()
         self.body_inertia = self.gravity = None
         self.inertia_bodies = ()
+        self.contact_friction = None
+        self.friction_constraints = ()
         why = C.c_char_p()
         if self._lib.arb_batch_step_path(self._batch_h, C.byref(why)) == 0:
             # not silent: the fused stages fold controllers per dof; anything else runs the
@@ -237,6 +239,39 @@ class BatchedWorld(object):
         g = None if gravity is False else self._device_f64(gravity, (3, self.nworlds), "gravity")
         _capi.check(self._lib, self._lib.arb_batch_bind_gravity(self._batch_h, g.data_ptr() if g is not None else None))
         self.gravity = g
+
+    # ---- per-world contact friction ------------------------------------------------------------
+    def contact_indices(self):
+        """constraint indices (registration order, as in ``arb_get_constraint``) of the soft-finger
+        contacts, the constraints whose friction ``set_contact_friction`` can bind"""
+        from .flatten import CONS_SOFT_FINGER
+        return [c for c, t in enumerate(np.asarray(self.model.cons_type).reshape(-1)) if int(t) == CONS_SOFT_FINGER]
+
+    def set_contact_friction(self, mu=None, constraints=None):
+        """Per-world friction coefficient of the contacts ``constraints`` (indices from
+        ``contact_indices()``): ``mu`` (len(constraints), W), in place of the model's ``_mu`` of that
+        contact in that world.  Numpy or torch; ``None`` keeps what is bound (``constraints`` too),
+        ``False`` unbinds.  The bound fp64 device tensor is ``contact_friction`` (the argument itself
+        when it already is one), its indices ``friction_constraints``: write into it in place to change
+        the friction between steps without another call."""
+        W = self.nworlds
+        p, cs = self.contact_friction, self.friction_constraints
+        if mu is False:
+            p, cs = None, ()
+        else:
+            if constraints is not None:
+                cs = tuple(int(c) for c in np.asarray(constraints).reshape(-1))
+            if mu is not None:
+                p = self._device_f64(mu, (len(cs), W), "mu")
+            elif p is not None and tuple(p.shape) != (len(cs), W):
+                raise ValueError("the bound mu has %d constraints, not %d: pass mu with its constraints"
+                                 % (p.shape[0], len(cs)))
+        ids = (C.c_int32*max(len(cs), 1))(*cs)
+        self._sync_stream()         # (the constraint table is replaced in stream order)
+        _capi.check(self._lib, self._lib.arb_batch_bind_contact_friction(
+            self._batch_h, len(cs) if p is not None else 0, ids, p.data_ptr() if p is not None else None))
+        self.contact_friction = p
+        self.friction_constraints = cs if p is not None else ()
 
     # ---- the four phases and the fused step ---------------------------------------------
     def update_dynamic(self):
@@ -454,7 +489,8 @@ class HostPipeline(object):
     ``gpos``, ``gvel``, ``cforce`` are C-contiguous (elem, W) numpy arrays over PINNED memory
     (e.g. ``torch.empty(...).pin_memory().numpy()``), updated in place.
     Every block is a batch of its own, so per-world inputs bound on one ``BatchedWorld``
-    (``set_controller_params``, ``set_applied_forces``, ``set_body_inertia``, ``set_gravity``) do not
+    (``set_controller_params``, ``set_applied_forces``, ``set_body_inertia``, ``set_gravity``,
+    ``set_contact_friction``) do not
     reach the pipeline: it steps the model's parameters."""
 
     def __init__(self, world_or_model, nworlds, chunks="auto", device=None, mode="serial",

@@ -164,6 +164,7 @@ extern "C" void arb_batch_destroy(arb_batch* b) {
   cudaFree(b->d.status);
   cudaFree(b->applied_rows);
   cudaFree(b->inertia_rows);
+  cudaFree(b->friction_rows);
   arb_fused_release(b);
   delete b;
 }
@@ -264,6 +265,24 @@ extern "C" int arb_batch_bind_gravity(arb_batch* b, const double* gravity) {
   return 0;
 }
 
+extern "C" int arb_batch_bind_contact_friction(arb_batch* b, int ncontacts, const int32_t* constraints, const double* mu) {
+  if (!b) { arb_set_error("null batch"); return -1; }
+  std::vector<int> rows;
+  std::string err;
+  if (friction_rows(b->model->host, ncontacts, constraints, mu != nullptr, rows, err)) {
+    arb_set_error(err);
+    return -1;
+  }
+  CUDA_OK(cudaSetDevice(b->device));
+  if (!b->friction_rows) CUDA_OK(cudaMalloc((void**)&b->friction_rows, sizeof(int) * rows.size()));
+  // in stream order: the steps already enqueued read the previous table
+  CUDA_OK(cudaMemcpyAsync(b->friction_rows, rows.data(), sizeof(int) * rows.size(), cudaMemcpyHostToDevice, b->stream));
+  CUDA_OK(cudaStreamSynchronize(b->stream));
+  b->friction.mu = ncontacts > 0 ? mu : nullptr;
+  b->friction.row = b->friction_rows;
+  return 0;
+}
+
 /* 1: arb_step runs the fused stages; 0: it runs the four phase kernels (a controller couples dofs
  * in a way the fused stages do not fold, or "force_phases" is set); *why (optional) names the reason */
 extern "C" int arb_batch_step_path(const arb_batch* b, const char** why) {
@@ -296,9 +315,12 @@ __global__ void __launch_bounds__(LPW_THREADS) k_update_controllers(DevModel m, 
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (w < b.W) world_update_controllers<PARAMS>(m, b, w, dt, ap);
 }
-__global__ void __launch_bounds__(LPW_THREADS) k_update_constraints(DevModel m, DevBatch b, double dt) {
+// FRIC: the instantiation with the world's contact friction, launched only while it is bound
+// (arb_batch_bind_contact_friction)
+template <bool FRIC>
+__global__ void __launch_bounds__(LPW_THREADS) k_update_constraints(DevModel m, DevBatch b, double dt, DevFriction fr) {
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (w < b.W) world_update_constraints(m, b, w, dt);
+  if (w < b.W) world_update_constraints<FRIC>(m, b, w, dt, fr);
 }
 __global__ void __launch_bounds__(LPW_THREADS) k_integrate(DevModel m, DevBatch b, double dt) {
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -315,6 +337,11 @@ static void launch_update_controllers(arb_batch* b, double dt) {
   if (params_bound(b))
     k_update_controllers<true><<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->applied);
   else k_update_controllers<false><<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->applied);
+}
+static void launch_update_constraints(arb_batch* b, double dt) {
+  if (b->friction.mu)
+    k_update_constraints<true><<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->friction);
+  else k_update_constraints<false><<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt, b->friction);
 }
 
 #define LAUNCH_CHECK(b)                                                        \
@@ -351,7 +378,7 @@ extern "C" int arb_update_constraints(arb_batch* b, double dt) {
   if (!(dt > 0)) { arb_set_error("dt must be > 0"); return -3; }
   CUDA_OK(cudaSetDevice(b->device));
   rc = arb_ensure_phase_scratch(b); if (rc) return rc;
-  k_update_constraints<<<lpw_grid(b->d.W), LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt);
+  launch_update_constraints(b, dt);
   LAUNCH_CHECK(b);
   b->last_fused = 0;
   return 0;
@@ -376,7 +403,7 @@ int arb_step_phases(arb_batch* b, const double* dts, int nsteps) {
     if (!(dt > 0)) { arb_set_error("dt must be > 0"); return -3; }
     launch_update_dynamic(b);
     launch_update_controllers(b, dt);
-    k_update_constraints<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt);
+    launch_update_constraints(b, dt);
     k_integrate<<<g, LPW_THREADS, 0, b->stream>>>(b->m, b->d, dt);
     b->launches += 3;
     LAUNCH_CHECK(b);

@@ -314,7 +314,11 @@ ARB_D int softfinger_solve(const double* v, const double* A, const double* P, do
   return 3;
 }
 
-ARB_D void world_update_constraints(const DevModel& m, const DevBatch& b, int64_t w, double dt) {
+// FRIC: the friction coefficients of the contacts in fr.row are the world's own
+// (arb_batch_bind_contact_friction, fr.mu); the instantiation launched only while they are bound
+template <bool FRIC = false>
+ARB_D void world_update_constraints(const DevModel& m, const DevBatch& b, int64_t w, double dt,
+                                    const DevFriction& fr = DevFriction{nullptr, nullptr}) {
   const int64_t W = b.W;
   const int n = m.ndof;
   int L = 0;
@@ -522,7 +526,12 @@ ARB_D void world_update_constraints(const DevModel& m, const DevBatch& b, int64_
             P4[4 * i + j] = AT(b.cpinv, r0 * 4 + 4 * i + j);
           }
         }
-        const int br = softfinger_solve(v, A4, P4, AT(b.caux, 4 * c), cd[36], cd + 37, dt, f, df, &status);
+        double mu = cd[36];
+        if constexpr (FRIC) {
+          const int row = fr.row[c];
+          if (row >= 0) mu = fr.mu[(int64_t)row * W + w];
+        }
+        const int br = softfinger_solve(v, A4, P4, AT(b.caux, 4 * c), mu, cd + 37, dt, f, df, &status);
 #pragma unroll
         for (int i = 0; i < 4; ++i) AT(b.cforce, r0 + i) = f[i];
         AT(b.cbranch, c) = br;

@@ -105,30 +105,33 @@ static void launch_prepare_lane(const arb_batch* b, const DevBatch& d, double dt
 #ifndef GS_THREADS
 #define GS_THREADS 128
 #endif
-template <int THREADS>
+// FRIC (every Gauss-Seidel kernel): the instantiation that reads the world's contact friction from
+// the scratch (world_friction_gather), launched only while it is bound
+template <int THREADS, bool FRIC>
 __global__ void __launch_bounds__(THREADS, GS_MINBLOCKS) k_fused_gs(DevModel m, DevBatch b, double dt) {
   FUSED_SLOT_WORLD();
   if (s >= b.W) return;
 #if GS_L_SMEM
   __shared__ double sL[36 * THREADS];
-  const unsigned long long key = world_fused_gs(m, fused_tile_view(b, s), w, dt, sL + threadIdx.x, THREADS);
+  const unsigned long long key = world_fused_gs<FRIC>(m, fused_tile_view(b, s), w, dt, sL + threadIdx.x, THREADS);
 #else
   double Lr[36];
-  const unsigned long long key = world_fused_gs(m, fused_tile_view(b, s), w, dt, Lr, 1);
+  const unsigned long long key = world_fused_gs<FRIC>(m, fused_tile_view(b, s), w, dt, Lr, 1);
 #endif
   if (b.fkey != nullptr) b.fkey[s] = key;
 }
 // Gauss-Seidel with the contact operands staged by TMA (world_fused_gs_staged): 10 KB of shared memory
 // and one mbarrier per warp, a 64-byte descriptor per constraint
-template <int THREADS, bool PLAIN>
+template <int THREADS, bool PLAIN, bool FRIC>
 __global__ void __launch_bounds__(THREADS, GS_MINBLOCKS) k_fused_gs_staged(DevModel m, DevBatch b, double dt) {
-  __shared__ __align__(128) double sbuf[(THREADS / 32) * (GS_STAGE_WARP_BYTES / 8)];
+  constexpr unsigned WARP_DBL = gs_stage_warp_bytes<FRIC>() / 8;
+  __shared__ __align__(128) double sbuf[(THREADS / 32) * WARP_DBL];
   __shared__ __align__(16) GsDesc sdesc[32];
   __shared__ __align__(8) unsigned long long sbar[THREADS / 32];
   __shared__ const double* swbase[THREADS / 32][5];
   const unsigned lane = threadIdx.x & 31u, wp = threadIdx.x >> 5;
   GsStage st;
-  st.buf = sbuf + wp * (GS_STAGE_WARP_BYTES / 8);
+  st.buf = sbuf + wp * WARP_DBL;
   st.buf_s = (unsigned)__cvta_generic_to_shared(st.buf);
   st.bar_s = (unsigned)__cvta_generic_to_shared(&sbar[wp]);
   st.parity = 0u;
@@ -152,18 +155,19 @@ __global__ void __launch_bounds__(THREADS, GS_MINBLOCKS) k_fused_gs_staged(DevMo
   const bool valid = s < b.W;
   const int64_t sv = valid ? s : b.W - 1;
   double Lr[36];
-  const unsigned long long key = world_fused_gs_staged<PLAIN>(m, fused_tile_view(b, sv), sv, valid, dt, Lr, 1, st);
+  const unsigned long long key = world_fused_gs_staged<PLAIN, FRIC>(m, fused_tile_view(b, sv), sv, valid, dt, Lr, 1, st);
   if (valid && b.fkey != nullptr) b.fkey[s] = key;
 }
-static void launch_gs(const arb_batch* b, const DevBatch& d, double dt) {
+template <bool FRIC>
+static void launch_gs_lane(const arb_batch* b, const DevBatch& d, double dt) {
   const int64_t W = d.W;
   const unsigned grid = (unsigned)((W + GS_THREADS - 1) / GS_THREADS);
   if (b->gs_stage && b->m.nc <= 32) {
-    if (b->gs_plain) k_fused_gs_staged<GS_THREADS, true><<<grid, GS_THREADS, 0, b->stream>>>(b->m, d, dt);
-    else k_fused_gs_staged<GS_THREADS, false><<<grid, GS_THREADS, 0, b->stream>>>(b->m, d, dt);
+    if (b->gs_plain) k_fused_gs_staged<GS_THREADS, true, FRIC><<<grid, GS_THREADS, 0, b->stream>>>(b->m, d, dt);
+    else k_fused_gs_staged<GS_THREADS, false, FRIC><<<grid, GS_THREADS, 0, b->stream>>>(b->m, d, dt);
   }
   else
-    k_fused_gs<GS_THREADS><<<grid, GS_THREADS, 0, b->stream>>>(b->m, d, dt);
+    k_fused_gs<GS_THREADS, FRIC><<<grid, GS_THREADS, 0, b->stream>>>(b->m, d, dt);
 }
 // block-cooperative Gauss-Seidel: the sliding-friction solves of a visit are pooled over the
 // block through shared memory (world_fused_gs_coop)
@@ -174,6 +178,7 @@ static void launch_gs(const arb_batch* b, const DevBatch& d, double dt) {
 #endif
 #define GS_COOP_SMEM (((ARB_SLIDE_NDBL + 4) * GS_COOP_CAP + 1) * sizeof(double) + \
                       (GS_COOP_CAP + 2) * sizeof(int))
+template <bool FRIC>
 __global__ void __launch_bounds__(GS_COOP_THREADS, GS_COOP_MINBLOCKS) k_fused_gs_coop(DevModel m, DevBatch b, double dt) {
   extern __shared__ double smem[];
   GsCoop co;
@@ -186,8 +191,34 @@ __global__ void __launch_bounds__(GS_COOP_THREADS, GS_COOP_MINBLOCKS) k_fused_gs
   FUSED_SLOT_WORLD();
   const bool valid = s < b.W;
   double Lr[36];     // cached Lambda_FF block: registers (shared memory would shrink the L1)
-  const unsigned long long key = world_fused_gs_coop(m, fused_tile_view(b, valid ? s : b.W - 1), w, valid, dt, co, Lr, 1);
+  const unsigned long long key = world_fused_gs_coop<FRIC>(m, fused_tile_view(b, valid ? s : b.W - 1), w, valid, dt, co, Lr, 1);
   if (valid && b.fkey != nullptr) b.fkey[s] = key;
+}
+
+// the world's contact friction into the scratch (world_friction_gather), read through perm like the
+// other per-world inputs
+__global__ void __launch_bounds__(256) k_friction_gather(DevModel m, DevBatch b, DevFriction fr) {
+  FUSED_SLOT_WORLD();
+  if (s < b.W) world_friction_gather(m, fused_tile_view(b, s), artic_param_world(b, w), fr);
+}
+
+// the Gauss-Seidel stage (after the prepare stage: the gather writes into the scratch the prepare
+// stage has just filled); with the friction instantiations only while friction is bound.  coop: the
+// gs_coop option applies (arb_step; arb_step_begin runs the per-lane kernels).  Returns the launches.
+static int launch_gs(arb_batch* b, const DevBatch& d, double dt, bool coop) {
+  const int64_t W = d.W;
+  const bool fric = b->friction.mu != nullptr;
+  if (fric) k_friction_gather<<<(unsigned)((W + 255) / 256), 256, 0, b->stream>>>(b->m, d, b->friction);
+  if (coop && b->m.nc <= 64 && b->gs_coop) {
+    const unsigned grid = (unsigned)((W + GS_COOP_THREADS - 1) / GS_COOP_THREADS);
+    if (fric) k_fused_gs_coop<true><<<grid, GS_COOP_THREADS, GS_COOP_SMEM, b->stream>>>(b->m, d, dt);
+    else k_fused_gs_coop<false><<<grid, GS_COOP_THREADS, GS_COOP_SMEM, b->stream>>>(b->m, d, dt);
+  } else if (fric) {
+    launch_gs_lane<true>(b, d, dt);
+  } else {
+    launch_gs_lane<false>(b, d, dt);
+  }
+  return fric ? 2 : 1;
 }
 
 __global__ void __launch_bounds__(FINISH_THREADS) k_fused_finish(DevModel m, DevBatch b, double dt) {
@@ -307,14 +338,18 @@ static int ensure_fused_scratch(arb_batch* b) {
     b->d.perm = f->perm[0];
     b->d.fkey = f->key[0];
   }
-  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs_coop, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GS_COOP_SMEM));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs_coop<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GS_COOP_SMEM));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs_coop<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GS_COOP_SMEM));
   if (group_supported(b))
     CUDA_OKF(cudaFuncSetAttribute(k_fused_prepare_group, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)group_smem_bytes(b)));
   // the per-lane stages live on L1 (operands re-read every sweep / pass): no shared-memory carve-out
-  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs<GS_THREADS>, cudaFuncAttributePreferredSharedMemoryCarveout, GS_L_SMEM ? 20 : GS_CARVEOUT));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs<GS_THREADS, false>, cudaFuncAttributePreferredSharedMemoryCarveout, GS_L_SMEM ? 20 : GS_CARVEOUT));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs<GS_THREADS, true>, cudaFuncAttributePreferredSharedMemoryCarveout, GS_L_SMEM ? 20 : GS_CARVEOUT));
   // (staged: 2 CTAs x 43 KB per SM; the driver rounds the carve-out up to the next configuration)
-  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs_staged<GS_THREADS, false>, cudaFuncAttributePreferredSharedMemoryCarveout, GS_STAGE_CARVEOUT));
-  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs_staged<GS_THREADS, true>, cudaFuncAttributePreferredSharedMemoryCarveout, GS_STAGE_CARVEOUT));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs_staged<GS_THREADS, false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, GS_STAGE_CARVEOUT));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs_staged<GS_THREADS, true, false>, cudaFuncAttributePreferredSharedMemoryCarveout, GS_STAGE_CARVEOUT));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs_staged<GS_THREADS, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, GS_STAGE_CARVEOUT));
+  CUDA_OKF(cudaFuncSetAttribute(k_fused_gs_staged<GS_THREADS, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, GS_STAGE_CARVEOUT));
   {   // the plain instantiation serves models of joint limits and contact-aligned one-body contacts only
     const HostModel& hm = b->model->host;
     bool plain = GS_STAGE_PLAIN != 0 && b->gs_plain_allow != 0;
@@ -461,17 +496,11 @@ int arb_fused_step(arb_batch* b, const double* dts, int nsteps) {
     else
       launch_prepare_lane(b, d, dt);
     if (ev[0]) cudaEventRecord(ev[1], b->stream);
-    if (b->m.nc > 0) {
-      if (b->m.nc <= 64 && b->gs_coop)
-        k_fused_gs_coop<<<(unsigned)((W + GS_COOP_THREADS - 1) / GS_COOP_THREADS), GS_COOP_THREADS,
-                          GS_COOP_SMEM, b->stream>>>(b->m, d, dt);
-      else
-        launch_gs(b, d, dt);
-    }
+    if (b->m.nc > 0) b->launches += launch_gs(b, d, dt, true);
     if (ev[0]) cudaEventRecord(ev[2], b->stream);
     if (grp) k_fused_finish_k<<<g, FUSED_THREADS, 0, b->stream>>>(b->m, d, dt);
     else k_fused_finish<<<(unsigned)((W + FINISH_THREADS - 1) / FINISH_THREADS), FINISH_THREADS, 0, b->stream>>>(b->m, d, dt);
-    b->launches += (b->m.nc > 0) ? 3 : 2;
+    b->launches += 2;
     ++f->steps;
     if (ev[0]) {   // diagnostic mode: per-stage device time of this step
       cudaEventRecord(ev[3], b->stream);
@@ -519,8 +548,8 @@ int arb_fused_step_half(arb_batch* b, double dt, int half) {
       k_fused_prepare_group<<<(unsigned)((W + GROUP_WPC - 1) / GROUP_WPC), GROUP_WPC * ARB_GL, group_smem_bytes(b), b->stream>>>(b->m, b->d, dt, 1);
     else
       launch_prepare_lane(b, b->d, dt);
-    if (b->m.nc > 0) launch_gs(b, b->d, dt);
-    b->launches += (b->m.nc > 0) ? 2 : 1;
+    if (b->m.nc > 0) b->launches += launch_gs(b, b->d, dt, false);
+    b->launches += 1;
   } else {
     if (b->half_group) k_fused_finish_k<<<g, FUSED_THREADS, 0, b->stream>>>(b->m, b->d, dt);
     else k_fused_finish<<<(unsigned)((W + FINISH_THREADS - 1) / FINISH_THREADS), FINISH_THREADS, 0, b->stream>>>(b->m, b->d, dt);

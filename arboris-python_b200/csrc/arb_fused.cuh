@@ -440,7 +440,9 @@ ARB_D void gs_cache_switch(const DevModel& m, const DevBatch& b, int64_t w, GsCa
 }
 
 // one visit of a constraint that touches TWO generator bodies (e.g. a ball-and-socket joint
-// between two moving bodies): everything through memory.
+// between two moving bodies): everything through memory.  FRIC: a contact's mu is the world's, in aux[2]
+// (world_friction_gather), not the model's.
+template <bool FRIC = false>
 ARB_NOINLINE void gs_visit_two_body(const DevModel& m, const DevBatch& b, int64_t w, int c, double dt, int* status) {
   const int NG = m.ngrows;
   const int type = m.ctype[c];
@@ -476,7 +478,8 @@ ARB_NOINLINE void gs_visit_two_body(const DevModel& m, const DevBatch& b, int64_
     double A4[16], P4[16];
 #pragma unroll
     for (int i = 0; i < 16; ++i) { A4[i] = FT(b.fAcc, r0 * 4 + i); P4[i] = FT(b.fP, r0 * 4 + i); }
-    const int br = softfinger_solve(v, A4, P4, FT(b.faux, 4 * c), cd[36], cd + 37, dt, f, df, status);
+    const double mu = FRIC ? FT(b.faux, 4 * c + 2) : cd[36];
+    const int br = softfinger_solve(v, A4, P4, FT(b.faux, 4 * c), mu, cd + 37, dt, f, df, status);
 #pragma unroll
     for (int i = 0; i < 4; ++i) FT(b.ff, r0 + i) = f[i];
     FT(b.fbranch, c) = br;
@@ -594,8 +597,8 @@ ARB_D int softfinger_solve_tiled(const double* v, const double* pA, const double
 
 // one visit of a constraint whose rows depend on ONE generator body (the other frame is on
 // the ground): ND rows, block in the cache
-// returns the solver branch (soft-finger contacts; 0 otherwise)
-template <int ND>
+// returns the solver branch (soft-finger contacts; 0 otherwise).  FRIC: mu from aux[2], as gs_visit_two_body.
+template <int ND, bool FRIC = false>
 ARB_D int gs_visit_one_body(const DevModel& m, const DevBatch& b, int64_t w, int c, double dt,
                             GsCache& k, int* status) {
   const double* cd = m.cdbl + ARB_CONS_NDBL * c;
@@ -637,7 +640,7 @@ ARB_D int gs_visit_one_body(const DevModel& m, const DevBatch& b, int64_t w, int
     }
   } else {
     br = softfinger_solve_tiled(v, b.fAcc + r0 * (4 * ARB_TILE), b.fP + r0 * (4 * ARB_TILE),
-                                paux[0], paux[ARB_TILE], cd[36], cd + 37, dt, f, df, status);
+                                paux[0], paux[ARB_TILE], FRIC ? paux[2 * ARB_TILE] : cd[36], cd + 37, dt, f, df, status);
 #pragma unroll
     for (int i = 0; i < ND; ++i) pf[i * ARB_TILE] = f[i];
     b.fbranch[c * ARB_TILE] = br;
@@ -940,6 +943,21 @@ ARB_D bool gs_world_nonfinite(const DevModel& m, const DevBatch& b) {
   for (int g = 0; g < NG; ++g) chk += FT(b.fv0, g) + FT(b.fLam, g * NG + g);
   return !isfinite(chk);
 }
+// Per-world friction (arb_batch_bind_contact_friction): the world's mu of every soft-finger contact,
+// or the model's where none is bound, into aux[2] of the contact's scratch, once per step between the
+// prepare and the Gauss-Seidel stage.  The sweeps then read mu by slot next to sdist (in the staged
+// kernel through the same bulk copy) instead of gathering it through perm at every visit.  wp: the
+// world's column in fr.mu.
+ARB_D void world_friction_gather(const DevModel& m, const DevBatch& b, int64_t wp, const DevFriction& fr) {
+  for (int c = 0; c < m.nc; ++c) {
+    if (m.ctype[c] != ARB_CONS_SOFT_FINGER_PLANE_POINT) continue;
+    const int row = fr.row[c];
+    FT(b.faux, 4 * c + 2) = row >= 0 ? arb_ld_state(fr.mu + (int64_t)row * b.W + wp) : m.cdbl[ARB_CONS_NDBL * c + 36];
+  }
+}
+
+// FRIC: the instantiation that reads each contact's mu from aux[2] (world_friction_gather)
+template <bool FRIC = false>
 ARB_D unsigned long long world_fused_gs(const DevModel& m, const DevBatch& b, int64_t w, double dt,
                                         double* Lstore, int Lstride) {
   const int NG = m.ngrows;
@@ -1013,10 +1031,10 @@ ARB_D unsigned long long world_fused_gs(const DevModel& m, const DevBatch& b, in
     if (type == ARB_CONS_JOINT_LIMITS) {
       gs_visit_limit(m, b, c, dt, k);
     } else if (gneed < 0) {
-      gs_visit_two_body(m, b, w, c, dt, &status);
+      gs_visit_two_body<FRIC>(m, b, w, c, dt, &status);
     } else {
       if (type == ARB_CONS_BALL_SOCKET) gs_visit_one_body<3>(m, b, w, c, dt, k, &status);
-      else if (gs_visit_one_body<4>(m, b, w, c, dt, k, &status) == 3 && c < 32) slid |= 1u << c;
+      else if (gs_visit_one_body<4, FRIC>(m, b, w, c, dt, k, &status) == 3 && c < 32) slid |= 1u << c;
 #ifdef ARB_HOSTTEST_COUNTERS
       if (arb_dbg_slidemask && c < 32 && FT(b.fbranch, c) == 3) arb_dbg_slidemask[w * ARB_GS_SWEEPS + sweep] |= 1u << c;
 #endif
@@ -1068,10 +1086,14 @@ struct GsDesc {           // one constraint, as the sweep loop needs it (shared 
 };
 #define GS_STAGE_AP_BYTES (2 * 16 * ARB_TILE * 8)      /* A_cc, pinv(A_cc) */
 #define GS_STAGE_T_BYTES (3 * ARB_TILE * 8)            /* t_c of an aligned contact, double-buffered */
-#define GS_STAGE_AUX_BYTES (2 * ARB_TILE * 8)          /* sdist, sdist / dt */
-#define GS_STAGE_WARP_BYTES (GS_STAGE_AP_BYTES + 2 * GS_STAGE_T_BYTES + GS_STAGE_AUX_BYTES)
+// aux rows: sdist, sdist / dt, and with FRIC the world's mu (world_friction_gather)
+template <bool FRIC> __host__ __device__ constexpr unsigned gs_stage_aux_rows() { return FRIC ? 3u : 2u; }
+template <bool FRIC> __host__ __device__ constexpr unsigned gs_stage_aux_bytes() { return gs_stage_aux_rows<FRIC>() * ARB_TILE * 8; }
+template <bool FRIC> __host__ __device__ constexpr unsigned gs_stage_warp_bytes() {
+  return GS_STAGE_AP_BYTES + 2 * GS_STAGE_T_BYTES + gs_stage_aux_bytes<FRIC>();
+}
 struct GsStage {
-  double* buf;          // the warp's staging buffer: A (16 rows of 32 lanes), P (16), aux (2), T (2 x 3)
+  double* buf;          // the warp's staging buffer: A (16 rows of 32 lanes), P (16), aux (2, or 3 with FRIC), T (2 x 3)
   unsigned buf_s;       // ... its shared-space address
   unsigned bar_s;       // shared-space address of the warp's mbarrier (one arrival per refill)
   unsigned parity;      // phase the next wait looks for (warp-uniform)
@@ -1087,16 +1109,18 @@ __device__ __forceinline__ void gs_bulk_g2s(unsigned dst_s, const double* src, u
 // refill for constraint c; tnext: the T buffer the visit of c will read.  One lane issues; the source
 // addresses come from the warp's tile pointers in shared memory (assembling them from the lane's own
 // view -- spilled 64-bit pointers minus the lane index -- was 95 instructions per visit, 7 % of the kernel's)
+template <bool FRIC>
 __device__ __forceinline__ void gs_stage_issue(const GsStage& st, int c, unsigned tnext) {
+  const unsigned AUXB = gs_stage_aux_bytes<FRIC>();
   const GsDesc& d = st.desc[c];
   const unsigned tb = d.aligned ? (unsigned)GS_STAGE_T_BYTES : 0u;
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;"
-               ::"r"(st.bar_s), "r"((unsigned)(GS_STAGE_AP_BYTES + GS_STAGE_AUX_BYTES) + tb) : "memory");
+               ::"r"(st.bar_s), "r"((unsigned)(GS_STAGE_AP_BYTES + AUXB) + tb) : "memory");
   gs_bulk_g2s(st.buf_s, st.wbase[0] + d.row * (4 * ARB_TILE), 16 * ARB_TILE * 8, st.bar_s);
   gs_bulk_g2s(st.buf_s + 16 * ARB_TILE * 8, st.wbase[1] + d.row * (4 * ARB_TILE), 16 * ARB_TILE * 8, st.bar_s);
-  gs_bulk_g2s(st.buf_s + GS_STAGE_AP_BYTES, st.wbase[2] + c * (4 * ARB_TILE), GS_STAGE_AUX_BYTES, st.bar_s);
+  gs_bulk_g2s(st.buf_s + GS_STAGE_AP_BYTES, st.wbase[2] + c * (4 * ARB_TILE), AUXB, st.bar_s);
   if (d.aligned)
-    gs_bulk_g2s(st.buf_s + GS_STAGE_AP_BYTES + GS_STAGE_AUX_BYTES + tnext * GS_STAGE_T_BYTES,
+    gs_bulk_g2s(st.buf_s + GS_STAGE_AP_BYTES + AUXB + tnext * GS_STAGE_T_BYTES,
                 st.wbase[d.g1 < 0 ? 4 : 3] + c * (24 * ARB_TILE), GS_STAGE_T_BYTES, st.bar_s);
 }
 __device__ __forceinline__ void gs_stage_wait(const GsStage& st) {
@@ -1165,8 +1189,10 @@ __device__ __forceinline__ int softfinger_begin_tiled(const double* v, const dou
 }
 
 // gs_visit_one_body<4> with staged operands.  vmask: the lanes of the warp that take part in this
-// visit (all of them are here); cn: the warp's next staged contact (-1: none left).
-template <bool PLAIN>
+// visit (all of them are here); cn: the warp's next staged contact (-1: none left).  FRIC: the lane's
+// own mu from the staged aux[2] instead of the descriptor's warp-uniform one; read before the refill
+// of the buffer, it is the one value of the operands held across the sliding solve.
+template <bool PLAIN, bool FRIC>
 __device__ __forceinline__ int gs_visit_contact_staged(const DevBatch& b, int c, double dt, GsCache& k, int* status,
                                                        const GsStage& st, unsigned vmask, int cn) {
   const GsDesc& d = st.desc[c];
@@ -1178,7 +1204,7 @@ __device__ __forceinline__ int gs_visit_contact_staged(const DevBatch& b, int c,
   const double* sA = st.buf + st.lane;
   const double* sP = sA + 16 * ARB_TILE;
   const double* sAux = sA + 32 * ARB_TILE;
-  const double* sT = sA + 34 * ARB_TILE + st.tsel * (3 * ARB_TILE);
+  const double* sT = sA + (32 + gs_stage_aux_rows<FRIC>()) * ARB_TILE + st.tsel * (3 * ARB_TILE);
   double v[4], f[4], df[4];
 #pragma unroll
   for (int i = 0; i < 4; ++i) f[i] = pf[i * ARB_TILE];
@@ -1195,11 +1221,12 @@ __device__ __forceinline__ int gs_visit_contact_staged(const DevBatch& b, int c,
     }
   }
   double A[16], alpha[4];
-  int br = softfinger_begin_tiled(v, sA, sP, sAux[0], sAux[ARB_TILE], d.mu, d.eps, dt, f, df, A, alpha);
+  const double mu = FRIC ? sAux[2 * ARB_TILE] : d.mu;
+  int br = softfinger_begin_tiled(v, sA, sP, sAux[0], sAux[ARB_TILE], mu, d.eps, dt, f, df, A, alpha);
   // every lane of the visit has read what it needs of A, P, aux: refill them (and the OTHER T buffer)
   // for the warp's next contact visit while this one's sliding solves run
   __syncwarp(vmask);
-  if (cn >= 0 && st.lane == (unsigned)(__ffs(vmask) - 1)) gs_stage_issue(st, cn, st.tsel ^ 1u);
+  if (cn >= 0 && st.lane == (unsigned)(__ffs(vmask) - 1)) gs_stage_issue<FRIC>(st, cn, st.tsel ^ 1u);
 #if GS_STAGE_PF_F
   // the forces of the next contact (written by this lane one sweep ago, read first thing in its visit):
   // into the L1 by an asynchronous copy to the dump row (arb_prefetch_l1)
@@ -1215,7 +1242,7 @@ __device__ __forceinline__ int gs_visit_contact_staged(const DevBatch& b, int c,
 #endif
   if (br == 3) {
     double newf[4];
-    softfinger_sliding(A, alpha, d.mu, d.eps, newf, status, slmask);
+    softfinger_sliding(A, alpha, FRIC ? mu : d.mu, d.eps, newf, status, slmask);
 #pragma unroll
     for (int i = 0; i < 4; ++i) { df[i] = newf[i] - f[i]; f[i] = newf[i]; }
   }
@@ -1267,7 +1294,8 @@ __device__ __forceinline__ void gs_desc_fill(const DevModel& m, GsDesc* desc, in
 // PLAIN: the model holds nothing but joint limits and contacts of contact-aligned bodies (human36 on a
 // ground plane): the instantiation without the general visits (ball-and-socket, two-body constraints,
 // 4x6 contact maps), whose code the sweep loop then does not carry through the instruction cache.
-template <bool PLAIN>
+// FRIC: the world's contact friction (world_friction_gather), staged with sdist.
+template <bool PLAIN, bool FRIC>
 __device__ unsigned long long world_fused_gs_staged(const DevModel& m, const DevBatch& b, int64_t w, bool valid, double dt,
                                                     double* Lstore, int Lstride, GsStage& st) {
   const unsigned FULL = 0xffffffffu;
@@ -1312,7 +1340,7 @@ __device__ unsigned long long world_fused_gs_staged(const DevModel& m, const Dev
   asm volatile("fence.proxy.async;" ::: "memory");
   __syncwarp();
   st.tsel = 0u;
-  if (wmask != 0u && st.lane == (unsigned)(__ffs(wlive) - 1)) gs_stage_issue(st, __ffs(wmask) - 1, 0u);
+  if (wmask != 0u && st.lane == (unsigned)(__ffs(wlive) - 1)) gs_stage_issue<FRIC>(st, __ffs(wmask) - 1, 0u);
   for (int sweep = 0; sweep < ARB_X_SWEEPS; ++sweep) {
     for (unsigned mm = wvis; mm != 0u; mm &= mm - 1u) {
       const int c = __ffs(mm) - 1;
@@ -1382,10 +1410,10 @@ __device__ unsigned long long world_fused_gs_staged(const DevModel& m, const Dev
         if (d.type == ARB_CONS_JOINT_LIMITS) {
           gs_visit_limit(m, b, c, dt, k);
         } else if (!PLAIN && d.gneed < 0) {
-          gs_visit_two_body(m, b, w, c, dt, &status);
+          gs_visit_two_body<FRIC>(m, b, w, c, dt, &status);
         } else if (!PLAIN && d.type == ARB_CONS_BALL_SOCKET) {
           gs_visit_one_body<3>(m, b, w, c, dt, k, &status);
-        } else if (gs_visit_contact_staged<PLAIN>(b, c, dt, k, &status, st, vmask, cn) == 3) {
+        } else if (gs_visit_contact_staged<PLAIN, FRIC>(b, c, dt, k, &status, st, vmask, cn) == 3) {
           slid |= 1u << c;
         }
       }
@@ -1463,7 +1491,9 @@ ARB_D void coop_solve_sliding(GsCoop& co, const double* eps) {
 }
 
 // soft-finger visit, part 1 (before the pooled solve): returns the branch (1 separating,
-// 2 static, 3 sliding: problem queued in *slot); f is updated for branches 1 and 2
+// 2 static, 3 sliding: problem queued in *slot); f is updated for branches 1 and 2.  FRIC: mu from
+// aux[2] (world_friction_gather); the queue carries it per problem either way.
+template <bool FRIC = false>
 ARB_D int gs_softfinger_begin(const DevModel& m, const DevBatch& b, int c, double dt, const GsCache& k,
                               GsCoop& co, double* f, double* df, int* slot, int* status) {
   const double* cd = m.cdbl + ARB_CONS_NDBL * c;
@@ -1475,7 +1505,7 @@ ARB_D int gs_softfinger_begin(const DevModel& m, const DevBatch& b, int c, doubl
   const double* pA = b.fAcc + r0 * (4 * ARB_TILE);
   const double* pP = b.fP + r0 * (4 * ARB_TILE);
   const double sdist = b.faux[c * (4 * ARB_TILE)];
-  const double mu = cd[36];
+  const double mu = FRIC ? b.faux[(c * 4 + 2) * ARB_TILE] : cd[36];
   const double* eps = cd + 37;
   double v[4], vnf[4];
   if (m.caligned[c]) {
@@ -1597,7 +1627,8 @@ ARB_D void gs_softfinger_end(const DevModel& m, const DevBatch& b, int c, GsCach
 }
 
 // `valid`: this thread has a world (w < W); threads without one only take part in the barriers.
-// Supports up to 64 constraints (the active set is a bit mask).
+// Supports up to 64 constraints (the active set is a bit mask).  FRIC: as world_fused_gs.
+template <bool FRIC = false>
 ARB_D unsigned long long world_fused_gs_coop(const DevModel& m, const DevBatch& b, int64_t w, bool valid,
                                              double dt, GsCoop& co, double* Lstore, int Lstride) {
   const int NG = m.ngrows;
@@ -1645,7 +1676,7 @@ ARB_D unsigned long long world_fused_gs_coop(const DevModel& m, const DevBatch& 
       if (g1 >= 0 && g0 >= 0) {
         if (act) {
           gs_cache_flush(m, b, w, k);
-          gs_visit_two_body(m, b, w, c, dt, &status);
+          gs_visit_two_body<FRIC>(m, b, w, c, dt, &status);
         }
         continue;
       }
@@ -1662,7 +1693,7 @@ ARB_D unsigned long long world_fused_gs_coop(const DevModel& m, const DevBatch& 
       int br = 0, slot = 0;
       if (act) {
         if (c + 1 < m.nc) gs_prefetch_visit(m, b, c + 1);
-        br = gs_softfinger_begin(m, b, c, dt, k, co, f, df, &slot, &status);
+        br = gs_softfinger_begin<FRIC>(m, b, c, dt, k, co, f, df, &slot, &status);
       }
       coop_solve_sliding(co, m.cdbl + ARB_CONS_NDBL * c + 37);
       if (act) gs_softfinger_end(m, b, c, k, co, br, slot, f, df, &status);

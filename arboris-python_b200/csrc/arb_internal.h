@@ -44,6 +44,8 @@ struct arb_batch {
   DevApplied applied = {nullptr, nullptr, nullptr};   // arb_batch_bind_applied_forces
   int* applied_rows = nullptr;     // device [nj]: applied.row (allocated on the first bind)
   int* inertia_rows = nullptr;     // device [nj]: applied.irow (arb_batch_bind_body_inertia, allocated on the first bind)
+  DevFriction friction = {nullptr, nullptr};   // arb_batch_bind_contact_friction
+  int* friction_rows = nullptr;    // device [nc]: friction.row (allocated on the first bind)
 };
 
 const char* arb_set_error(const std::string& s);

@@ -441,6 +441,25 @@ static inline int applied_wrench_rows(const HostModel& m, int nbodies, const int
   }
   return 0;
 }
+// Constraint -> mu row table of arb_batch_bind_contact_friction: rows[c] = i if constraints[i] == c,
+// else -1.  Refuses indices out of range, constraints that are not soft-finger contacts, duplicates
+// and mu without constraints.
+static inline int friction_rows(const HostModel& m, int ncontacts, const int32_t* constraints, bool has_mu,
+                                std::vector<int>& rows, std::string& err) {
+  if (ncontacts < 0) { err = "negative number of mu constraints"; return -1; }
+  if (ncontacts > 0 && !constraints) { err = "null constraint list"; return -1; }
+  if (has_mu && ncontacts == 0) { err = "a mu array needs its constraints"; return -1; }
+  rows.assign(m.nc > 0 ? m.nc : 1, -1);
+  for (int i = 0; i < ncontacts; ++i) {
+    const int c = constraints[i];
+    const std::string cs = std::to_string(c);
+    if (c < 0 || c >= m.nc) { err = "mu constraint " + cs + " out of range"; return -1; }
+    if (m.ctype[c] != ARB_CONS_SOFT_FINGER_PLANE_POINT) { err = "mu constraint " + cs + " is not a contact"; return -1; }
+    if (rows[c] >= 0) { err = "mu constraint " + cs + " listed twice"; return -1; }
+    rows[c] = i;
+  }
+  return 0;
+}
 
 // carve `dbl` (doubles) and `ints` into the DevBatch members; W worlds
 static inline void carve_scratch(const ScratchSizes& s, int64_t W, double* dbl, int* ints, DevBatch& b) {

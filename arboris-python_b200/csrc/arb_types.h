@@ -112,6 +112,15 @@ struct DevApplied {
   const double *gravity; // [3][W]        gravity in ground axes, in place of sum_a gravity_a up (caller-owned)
 };
 
+// Per-world friction coefficients of soft-finger contacts (arb_batch_bind_contact_friction), by WORLD
+// index; mu == nullptr: none.  The phase kernel reads them in its visits; the fused step gathers them
+// once per step into aux[2] of each contact's scratch (world_friction_gather), where the Gauss-Seidel
+// instantiations with FRIC find them.
+struct DevFriction {
+  const double *mu;      // [ncontacts][W] friction coefficient (caller-owned)
+  const int *row;        // [nc]          row of constraint c in mu, or -1: the model's (library-owned table)
+};
+
 // Per-batch memory: caller-owned state and the phase-API scratch are [elem][W]; the fused
 // scratch (f*, a*) is tiled [W/32][elem][32].
 struct DevBatch {

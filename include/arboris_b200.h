@@ -220,6 +220,24 @@ int arb_batch_bind_body_inertia(arb_batch *batch, int nbodies, const int32_t *bo
  * "prepare_group" option does not support them: arb_step / arb_step_begin return -1 while both are
  * set. */
 int arb_batch_bind_gravity(arb_batch *batch, const double *gravity);
+/* Per-world contact friction: the reference keeps one friction coefficient per soft-finger contact
+ * (SoftFingerContact._mu, constraints.py); a batch may give the contacts of every world their own.
+ *  mu          : DEVICE [ncontacts][W], caller-owned like the state, world index fastest: mu[i][w]
+ *                replaces _mu of contact constraints[i] in world w.
+ *  constraints : HOST list of ncontacts distinct constraint indices (registration order, as in
+ *                arb_get_constraint), each an ARB_CONS_SOFT_FINGER_PLANE_POINT; copied into a table of
+ *                the batch in stream order.
+ * NULL or ncontacts = 0 unbinds; -1 for an index out of range, a constraint that is not a contact, a
+ * duplicate index or mu without constraints (the previous binding is kept).  mu is read by WORLD index,
+ * whatever the thread assignment, at every step of arb_update_constraints, arb_step (fused stages and
+ * phase kernels), arb_step_begin and the host-buffer steps: write it in place, in stream order, to
+ * change it between calls.  The "prepare_group" option supports it.  eps (fixed at (1, 1, 1) by the
+ * reference, constraints.py:423) and the contact geometry stay the model's.
+ * The values are not checked.  The reference's sliding solve divides by mu, so the meaningful domain
+ * is finite mu > 0.  A NaN, or mu <= 0, stays confined to its own world: where it reaches the sliding
+ * solve it sets that world's ARB_STATUS_EIG_* bits (or ARB_STATUS_NONFINITE if the state goes
+ * non-finite); no other world's results change. */
+int arb_batch_bind_contact_friction(arb_batch *batch, int ncontacts, const int32_t *constraints, const double *mu);
 /* which implementation arb_step runs for this batch: 1 = the fused stages, 0 = the four phase
  * kernels (a PD controller with off-diagonal gains or two controllers on one dof -- Z then has
  * entries the per-dof articulated elimination does not fold -- or the "force_phases" option).
