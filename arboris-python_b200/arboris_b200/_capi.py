@@ -105,6 +105,8 @@ SYMBOLS = [
     ("arb_get_vector", _i32, [_vp, _i32, _vp, _i64, _i64]),
     ("arb_get_body", _i32, [_vp, _i32, _i32, _vp, _i64, _i64]),
     ("arb_get_constraint", _i32, [_vp, _i32, _vp, _i64, _i64]),
+    ("arb_get_fused", _i32, [_vp, _i32, _vp, _i64, _i64]),
+    ("arb_model_generators", _i32, [_vp, c_i32p, c_i32p, c_i32p, c_i32p, c_i32p, c_i32p]),
     ("arb_batch_status", _i32, [_vp, _vp]),
     ("arb_batch_launch_count", _i64, [_vp]),
     ("arb_batch_stage_ms", _i32, [_vp, c_dblp]),

@@ -409,6 +409,34 @@ class BatchedWorld(object):
                 self._batch_h, code, out.data_ptr(), w0, w1))
         return out
 
+    def generators(self):
+        """Generator layout of the fused stages (rows of ``fused()``): dict with ``body``, ``aligned``
+        and ``c0`` (one entry per generator body), ``limdof`` (one per joint-limit row) and ``ng``."""
+        ng, nrows = C.c_int32(), C.c_int32()
+        _capi.check(self._lib, self._lib.arb_model_generators(self._model_h, C.byref(ng), C.byref(nrows),
+                                                              None, None, None, None))
+        arr = [(C.c_int32*max(n, 1))() for n in (ng.value,)*3 + (nrows.value - 6*ng.value,)]
+        _capi.check(self._lib, self._lib.arb_model_generators(self._model_h, None, None, *arr))
+        body, aligned, c0, limdof = [[int(a[i]) for i in range(n)] for a, n in
+                                     zip(arr, (ng.value,)*3 + (nrows.value - 6*ng.value,))]
+        return {"body": body, "aligned": aligned, "c0": c0, "limdof": limdof, "ng": int(nrows.value)}
+
+    def fused(self, what, w0=0, w1=None):
+        """Diagnostic read-back of the fused prepare stage's hand-over (``arb_get_fused``), fp64:
+        ``qfree`` (W, ndof), ``v0`` (W, NG), ``lambda`` (W, NG, NG), ``gframe`` (W, ngen, 3, 3),
+        ``y`` (W, NG), ``delassus`` (W, nrows, 4), ``K`` (W, ndof, NG).  NaN where the world skipped
+        generator space (no active constraint)."""
+        w0, w1 = self._range(w0, w1)
+        g = self.generators()
+        ng, ngen, n = g["ng"], len(g["body"]), self.ndof
+        code, shape = {"qfree": (0, (n,)), "v0": (1, (ng,)), "lambda": (2, (ng, ng)),
+                       "gframe": (3, (ngen, 3, 3)), "y": (4, (ng,)),
+                       "delassus": (5, (int(self.model.nrows), 4)), "K": (6, (n, ng))}[what]
+        out = torch.full((w1 - w0,) + shape, float("nan"), dtype=torch.float64, device=self.device)
+        self._sync_stream()
+        _capi.check(self._lib, self._lib.arb_get_fused(self._batch_h, code, out.data_ptr(), w0, w1))
+        return out
+
     def status(self):
         """Per-world ARB_STATUS_* bits accumulated since the last call."""
         out = torch.zeros(self.nworlds, dtype=torch.int32, device=self.device)

@@ -2,6 +2,7 @@
 // sm_100a, fp64.  The fused step (lane-per-world stages, and the 16-lanes-per-world prepare stage of
 // arb_group.cuh) lives in arb_fused.cu.
 #include <cuda_runtime.h>
+#include <math_constants.h>
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -721,6 +722,83 @@ extern "C" int arb_get_constraint(arb_batch* b, int which, void* out, int64_t w0
   const int64_t tot = nw * cnt;
   k_gather_int<<<(unsigned)((tot + 255) / 256), 256, 0, b->stream>>>(src, (int*)out, cnt, b->d.W, w0, nw);
   LAUNCH_CHECK(b);
+  return 0;
+}
+
+// the fused hand-over of worlds [w0, w0 + nw): element e of the array `src` (a base pointer of the tiled
+// fused scratch), through the world -> slot map; NaN where generator space was skipped (no active
+// constraint, world_fused_prepare) and the identity for the frames of generator bodies that are not aligned
+__global__ void k_get_fused(DevModel m, DevBatch b, int which, const double* __restrict__ src, int cnt,
+                            double* __restrict__ out, int64_t w0, int64_t nw, const int* __restrict__ slots) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= nw * cnt) return;
+  const int64_t w = i / cnt;
+  const int e = (int)(i - w * cnt);
+  const int64_t s = slots ? (int64_t)slots[w0 + w] : w0 + w;
+  const int64_t tile = s / ARB_TILE, lane = s % ARB_TILE;
+  if (which == ARB_FUSED_GFRAME && !m.gen_aligned[e / 9]) {
+    out[i] = (e % 9) % 4 == 0 ? 1. : 0.;
+    return;
+  }
+  if (which != ARB_FUSED_QFREE && which != ARB_FUSED_GFRAME) {
+    const int* act = b.factive + tile * b.firec * ARB_TILE + lane;
+    bool any = false;
+    for (int c = 0; c < m.nc; ++c) any = any || act[c * ARB_TILE];
+    if (!any) {
+      out[i] = CUDART_NAN;
+      return;
+    }
+  }
+  out[i] = src[tile * b.frec * ARB_TILE + (int64_t)e * ARB_TILE + lane];
+}
+extern "C" int arb_get_fused(arb_batch* b, int which, double* out, int64_t w0, int64_t w1) {
+  if (!b || !out) { arb_set_error("null argument"); return -1; }
+  if (w0 < 0 || w1 > b->d.W || w0 >= w1) { arb_set_error("world range out of bounds"); return -1; }
+  if (!b->fused || !b->last_fused) {
+    arb_set_error("no fused hand-over to read: the last step ran the phase kernels, or no fused step was made");
+    return -1;
+  }
+  const DevModel& m = b->m;
+  const int NG = m.ngrows;
+  const double* src = nullptr;
+  int cnt = 0;
+  switch (which) {
+    case ARB_FUSED_QFREE: src = b->d.fq; cnt = m.ndof; break;
+    case ARB_FUSED_V0: src = b->d.fv0; cnt = NG; break;
+    case ARB_FUSED_LAMBDA: src = b->d.fLam; cnt = NG * NG; break;
+    case ARB_FUSED_GFRAME: src = b->d.fRe; cnt = 9 * m.ngen; break;
+    case ARB_FUSED_Y: src = b->d.fy; cnt = NG; break;
+    case ARB_FUSED_DELASSUS: src = b->d.fAcc; cnt = 4 * m.nrows; break;
+    case ARB_FUSED_K:
+      if (!b->last_group) {
+        arb_set_error("K = Z^-1 G^T is formed by the prepare_group prepare stage only, and the last step did not run it");
+        return -1;
+      }
+      src = b->d.fK; cnt = m.ndof * NG; break;
+    default: arb_set_error("unknown fused quantity"); return -1;
+  }
+  if (cnt == 0) return 0;
+  CUDA_OK(cudaSetDevice(b->device));
+  const int64_t nw = w1 - w0;
+  k_get_fused<<<(unsigned)((nw * cnt + 255) / 256), 256, 0, b->stream>>>(m, b->d, which, src, cnt, out, w0, nw,
+                                                                          arb_fused_world_slots(b));
+  LAUNCH_CHECK(b);
+  return 0;
+}
+
+extern "C" int arb_model_generators(const arb_model* model, int32_t* ngen, int32_t* ngrows, int32_t* gen_body,
+                                    int32_t* gen_aligned, int32_t* gen_c0, int32_t* glimdof) {
+  if (!model) { arb_set_error("null model"); return -1; }
+  const HostModel& h = model->host;
+  if (ngen) *ngen = h.ngen;
+  if (ngrows) *ngrows = h.ngrows;
+  for (int g = 0; g < h.ngen; ++g) {
+    if (gen_body) gen_body[g] = h.gen_body[g];
+    if (gen_aligned) gen_aligned[g] = h.gen_aligned[g];
+    if (gen_c0) gen_c0[g] = h.gen_c0[g];
+  }
+  if (glimdof)
+    for (size_t i = 0; i < h.glimdof.size(); ++i) glimdof[i] = h.glimdof[i];
   return 0;
 }
 

@@ -490,6 +490,7 @@ int arb_fused_step(arb_batch* b, const double* dts, int nsteps) {
       return leave(-3);
     }
     b->poses_valid = grp ? 0 : 1;      // (the group stage keeps poses on chip unless asked: arb_step_begin)
+    b->last_group = grp ? 1 : 0;
     if (ev[0]) cudaEventRecord(ev[0], b->stream);
     if (grp)
       k_fused_prepare_group<<<(unsigned)((W + GROUP_WPC - 1) / GROUP_WPC), GROUP_WPC * ARB_GL, group_smem_bytes(b), b->stream>>>(b->m, d, dt, 0);
@@ -543,6 +544,7 @@ int arb_fused_step_half(arb_batch* b, double dt, int half) {
   }
   if (half == 0) {
     b->half_group = grp ? 1 : 0;       // the finish half must match the prepare half
+    b->last_group = b->half_group;
     b->poses_valid = 1;
     if (grp)
       k_fused_prepare_group<<<(unsigned)((W + GROUP_WPC - 1) / GROUP_WPC), GROUP_WPC * ARB_GL, group_smem_bytes(b), b->stream>>>(b->m, b->d, dt, 1);

@@ -41,6 +41,7 @@ struct arb_batch {
   int half_open = 0;               // arb_step_begin ran the fused stages: arb_step_end must run the finish stage
   int prepare_group = 0;           // 1: prepare stage with 16 lanes per world and on-chip scratch (arb_group.cuh) + K-matrix finish
   int last_fused = 0;              // 1: the constraint read-backs come from the fused scratch (last step was fused)
+  int last_group = 0;              // 1: that step ran the group prepare stage (the scratch holds K, arb_get_fused)
   DevApplied applied = {nullptr, nullptr, nullptr};   // arb_batch_bind_applied_forces
   int* applied_rows = nullptr;     // device [nj]: applied.row (allocated on the first bind)
   int* inertia_rows = nullptr;     // device [nj]: applied.irow (arb_batch_bind_body_inertia, allocated on the first bind)

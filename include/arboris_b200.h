@@ -117,6 +117,21 @@ typedef enum {
                              homogeneousmatrix.py:225 (index work, bit-exact) */
 } arb_constraint_id;
 typedef enum { ARB_VEC_GFORCE = 0 } arb_vector_id;   /* World._gforce, core.py:665-667 */
+/* what the fused prepare stage hands to the Gauss-Seidel and finish stages (arb_get_fused); NG rows of
+ * "generator" space: 6 per generator body (its twist, in the frame R_e when contact-aligned), then one
+ * per joint-limit dof (arb_model_generators lists them) */
+typedef enum {
+  ARB_FUSED_QFREE = 0,    /* [ndof]      q_free = Z^-1 (M q'/dt + gforce), Z = M/dt + B + N + PD impedance */
+  ARB_FUSED_V0 = 1,       /* [NG]        G q_free */
+  ARB_FUSED_LAMBDA = 2,   /* [NG][NG]    G Z^-1 G^T, row-major as stored (Z is not symmetric, nor is this) */
+  ARB_FUSED_GFRAME = 3,   /* [ngen][9]   R_e = R_c^T R_body of the contact-aligned generator bodies, row-major;
+                             the identity for the others */
+  ARB_FUSED_Y = 4,        /* [NG]        wrench y = sum_c T_c^T f_c of the final constraint forces, what the
+                             finish stage solves with: q'+ = q_free + Z^-1 G^T y */
+  ARB_FUSED_DELASSUS = 5, /* [nrows][4]  diagonal Delassus block A_cc of every ACTIVE constraint, row-major
+                             d x d from element 4 crow[c] on (d = 1, 3 or 4 rows); other rows unspecified */
+  ARB_FUSED_K = 6         /* [ndof][NG]  K = Z^-1 G^T: the "prepare_group" prepare stage only */
+} arb_fused_id;
 
 /* per-world status bits (arb_batch_status) */
 #define ARB_STATUS_NONFINITE   1   /* NaN/Inf in gvel or gpos */
@@ -287,6 +302,20 @@ int arb_get_matrix(arb_batch *batch, int which, double *out, int64_t w0, int64_t
 int arb_get_vector(arb_batch *batch, int which, double *out, int64_t w0, int64_t w1);
 int arb_get_body(arb_batch *batch, int which, int body, double *out, int64_t w0, int64_t w1);
 int arb_get_constraint(arb_batch *batch, int which, void *out, int64_t w0, int64_t w1);
+/* Diagnostic read-back of the fused step's hand-over between its stages (arb_fused_id), fp64, for
+ * checking the prepare stage against a reference.  Valid after arb_step_begin and after an arb_step
+ * that ran the fused stages (then: of its last step, whose state the caller's arrays no longer hold);
+ * -1 with a message after a step through the phase kernels or before any fused step, and for
+ * ARB_FUSED_K unless that step ran the "prepare_group" stage.  A world with no active constraint skips
+ * generator space: V0, LAMBDA, Y, DELASSUS and K of such a world are NaN; QFREE and GFRAME are always
+ * formed.  Reads the scratch only: the step does no work for it. */
+int arb_get_fused(arb_batch *batch, int which, double *out, int64_t w0, int64_t w1);
+/* Generator layout of the model (the rows of arb_get_fused): *ngen generator bodies, *ngrows = NG rows.
+ * Each array may be NULL: gen_body[ngen] body index (1..njoints), gen_aligned[ngen] 1 if its rows are
+ * taken in the contact-aligned frame R_e, gen_c0[ngen] the contact whose plane normal defines R_e (-1 if
+ * not aligned), glimdof[NG - 6 ngen] the dof of each joint-limit row. */
+int arb_model_generators(const arb_model *model, int32_t *ngen, int32_t *ngrows, int32_t *gen_body,
+                         int32_t *gen_aligned, int32_t *gen_c0, int32_t *glimdof);
 /* int32 flags[W] (DEVICE), bits ARB_STATUS_*, accumulated since the last call */
 int arb_batch_status(arb_batch *batch, int32_t *flags);
 

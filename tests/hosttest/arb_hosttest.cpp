@@ -136,6 +136,58 @@ void ht_fused_step(void* p, double dt) {
     world_fused_finish(hb->dm, t, w, dt);
   }
 }
+// The prepare stage followed by the Gauss-Seidel's prologue only (diagonal Delassus blocks, the warm
+// start y0 = sum T_c^T f_c): the hand-over of the prepare stage without the sweeps, for
+// tests/test_prepare_reference.py (arb_hosttest_applied.cpp: the instantiation with applied forces).
+extern "C++" template <bool APPLIED, bool PARAMS>
+void fused_prepare_worlds(HostBatch* hb, double dt, const DevApplied& ap) {
+  for (int64_t w = 0; w < hb->b.W; ++w) {
+    const DevBatch b = fused_tile_view(hb->b, w);
+    world_fused_prepare<APPLIED, PARAMS>(hb->dm, b, w, dt, ap);
+    bool any = false;
+    for (int c = 0; c < hb->dm.nc; ++c) any = any || FT(b.factive, c);
+    for (int g = 0; g < hb->dm.ngrows; ++g) FT(b.fy, g) = 0.;
+    if (!any) continue;
+    for (int r = 0; r < hb->dm.nrows; ++r) FT(b.ff, r) = ST_LD(b.cforce, r);
+    gs_prologue(hb->dm, b, w, dt);
+  }
+}
+void ht_fused_prepare(void* p, double dt) {
+  fused_prepare_worlds<false, false>((HostBatch*)p, dt, DevApplied{nullptr, nullptr, nullptr});
+}
+// the finish stage alone, with the wrench y the caller left in fy (ht_fused_dbl_set)
+void ht_fused_finish(void* p, double dt) {
+  HostBatch* hb = (HostBatch*)p;
+  for (int64_t w = 0; w < hb->b.W; ++w) world_fused_finish(hb->dm, fused_tile_view(hb->b, w), w, dt);
+}
+static double* fused_dbl(HostBatch* hb, const std::string& s) {
+  const DevBatch& b = hb->b;
+  if (s == "fq") return b.fq; if (s == "fv0") return b.fv0; if (s == "fLam") return b.fLam;
+  if (s == "fRe") return b.fRe; if (s == "fy") return b.fy; if (s == "fAcc") return b.fAcc;
+  if (s == "adinv") return b.adinv;
+  return nullptr;
+}
+// fused double outputs are tiled: copied out as [elem][W] (ht_fused_dbl) or in from it (ht_fused_dbl_set)
+int ht_fused_dbl(void* p, const char* name, int nelem, double* out) {
+  HostBatch* hb = (HostBatch*)p;
+  const double* base = fused_dbl(hb, name);
+  if (!base) return -1;
+  for (int64_t w = 0; w < hb->b.W; ++w) {
+    const double* t = base + (w / ARB_TILE) * hb->b.frec * ARB_TILE + w % ARB_TILE;
+    for (int e = 0; e < nelem; ++e) out[e * hb->b.W + w] = t[e * ARB_TILE];
+  }
+  return 0;
+}
+int ht_fused_dbl_set(void* p, const char* name, int nelem, const double* in) {
+  HostBatch* hb = (HostBatch*)p;
+  double* base = fused_dbl(hb, name);
+  if (!base) return -1;
+  for (int64_t w = 0; w < hb->b.W; ++w) {
+    double* t = base + (w / ARB_TILE) * hb->b.frec * ARB_TILE + w % ARB_TILE;
+    for (int e = 0; e < nelem; ++e) t[e * ARB_TILE] = in[e * hb->b.W + w];
+  }
+  return 0;
+}
 // raw scratch access: which = index into the DevBatch double members in declaration order
 double* ht_array(void* p, const char* name) {
   HostBatch* hb = (HostBatch*)p;
@@ -212,6 +264,15 @@ int ht_aligned(void* p, int* flags, int* caligned) {
   for (int g = 0; g < hb->hm.ngen; ++g) flags[g] = hb->hm.gen_aligned[g];
   for (int c = 0; c < hb->hm.nc; ++c) caligned[c] = hb->hm.caligned[c];
   return hb->hm.ngen;
+}
+// generator layout: counts = {ngen, NG}; body, aligned, c0 [ngen]; limdof [NG - 6 ngen] (NULL: counts only)
+void ht_generators(void* p, int* counts, int* body, int* aligned, int* c0, int* limdof) {
+  const HostModel& h = ((HostBatch*)p)->hm;
+  counts[0] = h.ngen;
+  counts[1] = h.ngrows;
+  if (!body) return;     // counts only
+  for (int g = 0; g < h.ngen; ++g) { body[g] = h.gen_body[g]; aligned[g] = h.gen_aligned[g]; c0[g] = h.gen_c0[g]; }
+  for (size_t i = 0; i < h.glimdof.size(); ++i) limdof[i] = h.glimdof[i];
 }
 int ht_solve4(const double* a, const double* b, double* x) { return solve_small<4>(a, b, x) ? 1 : 0; }
 void ht_exp(const double* tw, double* out12) {

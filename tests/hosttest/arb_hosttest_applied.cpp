@@ -60,4 +60,10 @@ void ht_applied_fused_step(void* p, double dt) {
     world_fused_finish(hb->dm, t, w, dt);
   }
 }
+// the prepare stage + Gauss-Seidel prologue (ht_fused_prepare) with the instantiation the device picks
+void ht_applied_fused_prepare(void* p, double dt) {
+  const DevApplied ap = g_applied[p].ap;
+  if (ap.tau || ap.wrench) fused_prepare_worlds<true, false>((HostBatch*)p, dt, ap);
+  else fused_prepare_worlds<false, false>((HostBatch*)p, dt, ap);
+}
 }
